@@ -6,12 +6,16 @@ palette + Gilbert dither) on batches of synthetic 4K images, one process per GPU
   python bench.py --impl reference ...                     the CPU arm: the oracle (C++ restatement of
                                                            the reference's Java core; no JVM exists here)
                                                            on all host cores, rank 0 only
+  python bench.py ... --dump-outputs DIR                   also writes the output images of the last timed
+                                                           step (a fixed, seeded sample of them) to DIR/*.npy
 
 A step is one pass of convert() over this rank's batch of images. `value` is measured with the
 pixels already resident in HBM (nq_convert_batch_device), `e2e` through the host-buffer entry point
 (nq_convert_batch: pinned host -> device -> host inside the timed region). The headline line is weak
 scaling (every rank owns `--batch` images: BASELINE.json configs[3], 1024 x 4K, at N = 1); for N > 1 the
 same run also times configs[3]'s fixed batch split over the ranks (`strong`). Prints ONE JSON line on rank 0.
+`value` times exactly --steps steps; the `strong` and `e2e` legs time min(--steps, 5) steps of their own
+and report that number as their `steps`.
 """
 import argparse
 import json
@@ -42,12 +46,17 @@ try:   # per-kernel DRAM bytes per pixel from this round's `ncu --set full` capt
     NCU_DRAM_BYTES_PER_PIXEL.update(json.load(open(os.path.join(HERE, "profiles", "ncu_dram_bytes_per_pixel.json"))))
 except Exception:
     pass
+# --dump-outputs: at most this many output pixels per run (4 float32 channels, 16 bytes each: 32 MiB), sampled with DUMP_SEED
+# beyond that
+DUMP_PIXELS = 1 << 21
+DUMP_SEED = 0x0DD5EED
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps of the headline measurement; the strong and e2e legs time min(steps, 5)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=int(os.environ.get("NQ_BENCH_BATCH", "1024")),
@@ -70,7 +79,16 @@ def parse():
     ap.add_argument("--cpu-workers", type=int, default=0, help="reference arm: worker processes (0 = all cores)")
     ap.add_argument("--cpu-width", type=int, default=0, help="CPU legs: width of the sample image (0 = the workload's own)")
     ap.add_argument("--cpu-height", type=int, default=0, help="CPU legs: height of the sample image (0 = the workload's own)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output pixels of the last step to DIR/output_argb.npy (float32, one row "
+                         f"of A, R, G, B per pixel; batches of more than {DUMP_PIXELS} pixels per run: a sample at positions drawn "
+                         "from a fixed seed)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs: it needs --impl ours")
+    return a
 
 
 def workload_quantizer(a):
@@ -221,6 +239,25 @@ def _golden_check(a, ctx, din, dout, n, rank, seeds):
     return {"case": "config3_4k_lab_img0", "output_matches_oracle": got == c["output_sha"]}
 
 
+def dump_outputs(a, dout, rank, world):
+    """--dump-outputs: the ARGB images the device path wrote to `dout` (what its caller receives), one row (A, R, G, B) of
+    float32 channel values 0..255 per pixel, so that a tolerance on the values is a tolerance on colour. Above DUMP_PIXELS
+    pixels per run, the pixels at DUMP_PIXELS flat positions of the batch, drawn with DUMP_SEED and sorted: the same positions
+    on every run with the same arguments. One file per rank."""
+    import torch
+    budget = DUMP_PIXELS // world
+    total = dout.numel()
+    if total <= budget:
+        vals = dout
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(total, budget, replace=False))
+        vals = dout[torch.from_numpy(idx).to(dout.device)]
+    os.makedirs(a.dump_outputs, exist_ok=True)
+    name = "output_argb.npy" if world == 1 else f"output_argb_rank{rank}.npy"
+    argb = vals.cpu().numpy().view(np.uint32)
+    np.save(os.path.join(a.dump_outputs, name), np.stack([(argb >> s) & 255 for s in (24, 16, 8, 0)], axis=1).astype(np.float32))
+
+
 def run_ours(a, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -284,6 +321,8 @@ def run_ours(a, rank, world, local_rank):
     ms_max = max_over_ranks(ms)
     total_px = world * n * npix * a.steps
     value = total_px / (ms_max / 1e3) / 1e6
+    if a.dump_outputs:
+        dump_outputs(a, dout, rank, world)
 
     # ---- BASELINE.json configs[3] as written: ONE batch of --strong-batch images split over the ranks (N > 1 only; at N = 1
     #      it is the headline line itself when --batch equals it)
