@@ -149,6 +149,9 @@ typedef struct nq_image_info {
   /* FIFO dither kernel: SM cycles of the serial (consumer) warp, of which waiting for the producer warp, and cycles the
      producer warp waited for ring space */
   unsigned long long dither_cycles[3];
+  /* CIELAB merge loop: rounds of rescans (stale heap entries rescanned together, see nq_pnn.cuh), and rescans computed
+     in a round but not applied because a merge or the next round came first. `rescans` counts the applied ones only. */
+  unsigned long long merge_rounds, rescans_discarded;
 } nq_image_info;
 int nq_get_image_info(nq_ctx* ctx, int image, nq_image_info* out);
 /* sizeof(nq_image_info) as the library was built: lets a binding check its own mirror of the struct. */

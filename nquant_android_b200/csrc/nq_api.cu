@@ -183,8 +183,6 @@ struct nq_ctx {
   unsigned long long launches = 0;
   bool debug = false;
   int chunkImages = 0;                // images per chunk (0 = automatic)
-  int mergeRot = 0;                   // NQ_MERGE_ROT=1: rotate the logical warp ids of the merge kernels by the CTA index (measured: no
-                                      // effect, the hardware already spreads the warps of co-resident CTAs over the schedulers)
   // Gilbert orders by (w,h), least recently used first in orderLru
   std::map<std::pair<int, int>, uint32_t*> orders;
   std::vector<std::pair<int, int>> orderLru;
@@ -661,9 +659,9 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
     int* live = c->dLive + (size_t)ch.base * NQ_NBINS;
     int* pos = c->dPos + (size_t)ch.base * NQ_NBINS;
     if (kind == NQ_KIND_RGB) {
-      nq::k_merge_rgb<<<n, NQ_RGB_THREADS, (size_t)NQ_RGB_HEAP_SMEM * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0, c->mergeRot); ++c->launches;
+      nq::k_merge_rgb<<<n, NQ_RGB_THREADS, (size_t)NQ_RGB_HEAP_SMEM * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0); ++c->launches;
     } else {
-      nq::k_merge_lab<<<n, NQ_LAB_THREADS, (size_t)NQ_LAB_HEAP_SMEM * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0, c->mergeRot); ++c->launches;
+      nq::k_merge_lab<<<n, NQ_LAB_THREADS, (size_t)NQ_LAB_HEAP_SMEM * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0); ++c->launches;
     }
   } else { mark(2); mark(3); }
   mark(4);
@@ -988,7 +986,6 @@ nq_ctx* nq_create(int device) {
   }
   if (const char* e = getenv("NQ_SPEC_SLOTS")) c->specSlotsMax = atoi(e);
   if (const char* e = getenv("NQ_SPEC_POOL_GB")) c->specPoolMaxBytes = (size_t)atoi(e) << 30;
-  if (const char* e = getenv("NQ_MERGE_ROT")) c->mergeRot = atoi(e) != 0;
   bool haveLut = false;
   {
     DevBuf dBn, dW;
@@ -1166,6 +1163,7 @@ int nq_get_image_info(nq_ctx* c, int image, nq_image_info* o) {
   o->full_evals = I.statFullEvals;
   for (int k = 0; k < 6; ++k) o->merge_cycles[k] = I.statCyc[k];
   o->live_blocks = I.statLiveBlocks; o->screened = I.statScreened;
+  o->merge_rounds = I.statRounds; o->rescans_discarded = I.statDiscarded;
   for (int k = 0; k < 3; ++k) o->dither_cycles[k] = I.statDither[k];
   o->error = I.error;
   return NQ_OK;

@@ -485,10 +485,22 @@ __device__ __forceinline__ unsigned pack_idnn(int id, int nn) { return (unsigned
 //   4. the screened bins are evaluated in full, packed one per thread, and resolved in list order.
 // Every test is the reference's test against an err that is >= the err the sequential scan would hold
 // at that candidate, so nothing the reference would take is dropped, and step 4 replays its decisions.
-// 128 threads and 48 KB of heap per CTA: several images share an SM and fill each other's serial gaps.
+//
+// Rescans run in ROUNDS of up to NQ_LAB_ROUND bins. Between two merges the reference pops the heap top,
+// rescans it if it is stale and pushes it down, until the top is valid (PL:271-293). A rescan of bin b is a
+// pure function of b and the set of live bins, and it changes the validity of no other bin, so the bins it
+// rescans before the next merge are the stale entries in the order the heap pops them, up to the first valid
+// one. A round guesses them from the top levels of the heap (stale entries in ascending (err, slot), deleted
+// ones skipped, none behind a valid one) and rescans them together: step 1 takes one warp per bin, and steps
+// 2-4 run over all of them at once, batch g holding the g-th 32 live blocks of every bin, so that each bin is
+// pruned on the schedule of a rescan of its own. Thread 0 then replays the reference's top loop verbatim: a stale top with a result from the current
+// round takes it, one without starts the next round, and a merge discards the unused results. A wrong guess
+// costs work, never a different result.
+// 128 threads and 44 KB of heap per CTA: several images share an SM and fill each other's serial gaps.
 // -------------------------------------------------------------------------------------------------
 #define NQ_LAB_THREADS 128
 #define NQ_LAB_HEAP_SMEM 5632   // 44 KB of heap: four CTAs fit one SM
+#define NQ_LAB_ROUND 4          // bins rescanned together in one round (8 would need 256-entry batches: more shared memory)
 
 __device__ __forceinline__ int block_excl_scan_128(int v, int* total, int* sScan /*[8]*/) {
   const unsigned lane = lane_id(), w = threadIdx.x >> 5;
@@ -539,36 +551,41 @@ __device__ __forceinline__ int rebuild_live_lab(const NqSlot& S, const LabScratc
   return total;
 }
 
-__global__ void __launch_bounds__(NQ_LAB_THREADS, 4) k_merge_lab(NqImage* imgs, const NqSlot* slots, int* liveBuf, int* posBuf, int logMerges, int rot) {
+__global__ void __launch_bounds__(NQ_LAB_THREADS, 4) k_merge_lab(NqImage* imgs, const NqSlot* slots, int* liveBuf, int* posBuf, int logMerges) {
+  constexpr int R = NQ_LAB_ROUND;
+  static_assert(R >= 1 && 32 * R <= NQ_LAB_THREADS, "a batch holds 32 blocks of each bin of the round, one per thread");
   extern __shared__ unsigned char smemRaw[];
   float* sErr = reinterpret_cast<float*>(smemRaw);
   unsigned* sId = reinterpret_cast<unsigned*>(smemRaw + (size_t)NQ_LAB_HEAP_SMEM * 4);
   __shared__ int sScan[8];
-  __shared__ unsigned sBits[64];             // live blocks of this rescan, one bit per block
-  __shared__ unsigned short sBlk[2048];      // the same as an ordered list
-  __shared__ unsigned sMaskA[32];            // bins that passed the cheap bound, per block of the current batch
-  __shared__ unsigned sMaskB[32];            // ... of those, the ones that passed the screen, per 32 list entries
-  __shared__ int sOffA[33], sOffB[33];
+  __shared__ unsigned sBits[R][64];          // live blocks of each bin of the round, one bit per block
+  __shared__ unsigned short sPre[R][65];     // live blocks of the bin before each word of sBits; [64]: all of them
+  __shared__ unsigned short sBat[NQ_LAB_THREADS];   // entries of the current batch: bin of the round << 11 | block, bin-major
+  __shared__ unsigned sMaskA[NQ_LAB_THREADS];       // bins that passed the cheap bound, per entry of the batch
+  __shared__ unsigned sMaskB[NQ_LAB_THREADS];       // ... of those, the ones that passed the screen, per 32 of them
+  __shared__ int sOffA[NQ_LAB_THREADS + 1], sOffB[NQ_LAB_THREADS];
   __shared__ double sGs[NQ_LAB_THREADS], sGw[NQ_LAB_THREADS], sF[NQ_LAB_THREADS];
-  __shared__ int sPos[NQ_LAB_THREADS];       // position of a fully evaluated survivor, -1 = rejected
-  __shared__ double sErrCur;
-  __shared__ int sNnCur, sAction, sB1, sHeapN, sIter, sNLive;
+  __shared__ int sPos[NQ_LAB_THREADS];       // fully evaluated candidate: bin of the round << 17 | survived << 16 | position
+  // the round: bin ids, probes, running err and nn of each (nn: position in the live list while the round runs, bin id
+  // after it), first candidate position
+  __shared__ LabProbe sProbe[R];
+  __shared__ double sErrR[R];
+  __shared__ int sBinR[R], sNnR[R], sFirstR[R];
+  __shared__ int sAction, sB1, sHeapN, sIter, sNRound;
 
   const int img = blockIdx.x;
   NqImage& I = imgs[img];
   if (I.kind != NQ_KIND_LAB || I.nmax <= 2 || I.skipPnn) return;
   const NqSlot& S = slots[img];
   const LabScratch X = lab_scratch(S);
-  // The serial phases (heap top, ordered replay) belong to logical warp 0. Several CTAs share an SM, and the hardware
-  // places warp k of every CTA on the same scheduler: rotating the logical warp ids by the CTA index spreads the serial
-  // warps of co-resident images over the four schedulers.
-  const int t = (int)((threadIdx.x + 32u * (rot ? (blockIdx.x & 3u) : 0u)) & 127u);
+  const int t = threadIdx.x;
   const unsigned lane = lane_id(), w = t >> 5;
   const int W = NQ_LAB_THREADS / 32;
   const int maxbins = I.maxbins, extbins = I.extbins;
   int* live = liveBuf + (size_t)img * NQ_NBINS;
   int* posOf = posBuf + (size_t)img * NQ_NBINS;
   HeapView<NQ_LAB_HEAP_SMEM> H{sErr, sId, S.heap};
+  const float4 dead = make_float4(-1.f, 0.f, 0.f, 0.f);
 
   // ---- heap build: sequential pushes in bin order (PL:246-257), replayed by warp 0
   if (w == 0) {
@@ -592,196 +609,274 @@ __global__ void __launch_bounds__(NQ_LAB_THREADS, 4) k_merge_lab(NqImage* imgs, 
         __syncwarp();
       }
     }
-    if (lane == 0) { sHeapN = heapN; sIter = 0; }
+    if (lane == 0) { sHeapN = heapN; sIter = 0; sNRound = 0; }
   }
   __syncthreads();
   int liveLen = rebuild_live_lab(S, X, maxbins, live, posOf, sScan);
   int liveAtRebuild = liveLen, iterAtRebuild = 0;
-  unsigned long long rescans = 0, pairs = 0, fulls = 0, liveBlocks = 0, screened = 0;
+  unsigned long long rescans = 0, pairs = 0, fulls = 0, liveBlocks = 0, screened = 0, rounds = 0, discarded = 0;
   unsigned pops = 0;
+  unsigned used = 0;                           // thread 0: results of the current round applied so far, one bit per bin
   const double ratioMerge = I.ratioMerge;
   long long cyc[6] = {0, 0, 0, 0, 0, 0};
   long long tk = clock64();
   auto tick = [&](int k) { const long long now = clock64(); cyc[k] += now - tk; tk = now; };
 
   for (;;) {
-    // ---- thread 0: look at the heap top (PL:271-283)
-    if (t == 0) {
-      int action = 0;  // 0 = merge, 1 = rescan, 2 = finished
-      if (sIter >= extbins) action = 2;
-      else {
-        int heapN = sHeapN;
-        for (;;) {
-          const unsigned top = H.idnn(1);
-          int b1 = (int)(top & 0xFFFFu);
-          const int tm = S.bTm[b1], mtm = S.bMtm[b1], nmtm = S.bMtm[top >> 16];   // three independent loads
-          if (tm >= mtm && nmtm <= tm) { action = 0; sB1 = b1; break; }
-          if (mtm == NQ_DELETED) {
-            const unsigned last = H.idnn(heapN);
-            float e1 = H.err(heapN);
-            --heapN;
-            ++pops;
-            H.sift_down(last, e1, heapN);
-            continue;
+    if (w == 0) {
+      // ---- thread 0: the reference's top loop (PL:271-293); a stale top takes its result from the current round
+      if (lane == 0) {
+        int action = 0;  // 0 = merge, 1 = new round, 2 = finished
+        if (sIter >= extbins) action = 2;
+        else {
+          int heapN = sHeapN;
+          const int nRound = sNRound;
+          for (;;) {
+            const unsigned top = H.idnn(1);
+            const int b1 = (int)(top & 0xFFFFu);
+            const int tm = S.bTm[b1], mtm = S.bMtm[b1], nmtm = S.bMtm[top >> 16];   // three independent loads
+            if (tm >= mtm && nmtm <= tm) { action = 0; sB1 = b1; break; }
+            if (mtm == NQ_DELETED) {
+              const unsigned last = H.idnn(heapN);
+              float e1 = H.err(heapN);
+              --heapN;
+              ++pops;
+              H.sift_down(last, e1, heapN);
+              continue;
+            }
+            int j = 0;
+            while (j < nRound && sBinR[j] != b1) ++j;
+            if (j == nRound) { action = 1; break; }
+            // tb.tm = i; push slot down (PL:281-293)
+            const float e1 = (float)sErrR[j];
+            const int nnBin = sNnR[j];
+            S.bErr[b1] = e1; S.bNn[b1] = nnBin; S.bTm[b1] = sIter;
+            H.sift_down(pack_idnn(b1, nnBin), e1, heapN);
+            ++rescans;
+            used |= 1u << j;
+            pairs += (unsigned long long)max(0, liveLen - sFirstR[j]);
           }
-          action = 1; sB1 = b1;
-          break;
+          sHeapN = heapN;
+          if (action != 2) {                   // a merge or a new round: the results not applied are dropped
+            discarded += (unsigned long long)__popc(~used & (nRound == 32 ? ~0u : (1u << nRound) - 1u));
+            used = 0;
+            sNRound = 0;
+            rounds += action == 1;
+          }
         }
-        sHeapN = heapN;
+        sAction = action;
       }
-      sAction = action;
+      __syncwarp();
+      // ---- warp 0: choose the round from heap slots 1..32 (all in shared memory), one entry per lane. The stale
+      // entries ahead of the first valid one in (err, slot) order, deleted ones skipped, at most R of them; the
+      // stale top is the first. Deeper entries are never smaller than their ancestors, so the order is the heap's
+      // own for the first entries of the window; beyond them it is a guess, which only costs work if wrong.
+      if (sAction == 1) {
+        const int l = 1 + (int)lane;
+        float e = 0.f;
+        int b = 0;
+        bool valid = false, stale = false;
+        if (l <= sHeapN) {
+          const unsigned v = H.idnn(l);
+          e = H.err(l); b = (int)(v & 0xFFFFu);
+          const int tm = S.bTm[b], mtm = S.bMtm[b], nmtm = S.bMtm[v >> 16];
+          valid = tm >= mtm && nmtm <= tm;
+          stale = !valid && mtm != NQ_DELETED;
+        }
+        float ve = valid ? e : INFINITY;
+#pragma unroll
+        for (int o = 16; o; o >>= 1) ve = fminf(ve, __shfl_xor_sync(0xffffffffu, ve, o));
+        const unsigned vm = __ballot_sync(0xffffffffu, valid && e == ve);
+        const int lv = vm ? __ffs(vm) - 1 : 32;                  // the first valid entry
+        const bool cand = stale && (e < ve || (e == ve && (int)lane < lv));
+        const unsigned cm = __ballot_sync(0xffffffffu, cand);
+        int rank = 0;
+#pragma unroll
+        for (int k = 0; k < 32; ++k) {
+          const float ek = __shfl_sync(0xffffffffu, e, k);
+          rank += ((cm >> k) & 1u) && (ek < e || (ek == e && k < (int)lane));
+        }
+        if (cand && rank < R) sBinR[rank] = b;
+        if (lane == 0) sNRound = min(R, __popc(cm));
+      }
     }
-    if (t < 64) sBits[t] = 0u;
     __syncthreads();
     tick(0);
     const int action = sAction;
     if (action == 2) break;
-    const int b1 = sB1;
 
     if (action == 1) {
-      ++rescans;
-      const int first = posOf[b1] + 1;
+      const int n = sNRound;
       const LabView V{X.q, X.al, X.bs, liveLen};
-      const LabProbe P = lab_probe(I, S, b1, ratioMerge);
-      double err = 1e100;
-      int nn = -1;                              // position in the live list
-      // -- 1. the first 32 candidates in full
-      if (w == 0) {
+      for (int k = t; k < R * 64; k += NQ_LAB_THREADS) (&sBits[0][0])[k] = 0u;
+      // -- 1. the first 32 candidates of each bin in full, one warp per bin
+      for (int j = (int)w; j < n; j += W) {
+        const int b = sBinR[j];
+        const LabProbe P = lab_probe(I, S, b, ratioMerge);
+        const int first = posOf[b] + 1;
+        double err = 1e100;
+        int nn = -1;                            // position in the live list
         const int i = first + (int)lane;
         LabCand c;
         const bool alive = i < liveLen && lab_eval_t<false>(P, V, i, err, &c);
         lab_accept_in_order(alive, c, i, err, nn);
         fulls += i < liveLen;
-        if (lane == 0) { sErrCur = err; sNnCur = nn; }
+        if (lane == 0) { sProbe[j] = P; sErrR[j] = err; sNnR[j] = nn; sFirstR[j] = first; }
       }
       __syncthreads();
       tick(1);
-      err = sErrCur; nn = sNnCur;
-      // -- 2. block summaries of everything behind them
-      const int stop = first + 32;
-      const int blkBeg = stop >> 5, nblk = (liveLen + 31) >> 5;
-      for (int blk = blkBeg + t; blk < nblk; blk += NQ_LAB_THREADS)
-        if (!lab_block_skip(P, V, blk, err)) atomicOr(&sBits[blk >> 5], 1u << (blk & 31));
+      // -- 2. block summaries of everything behind them, the blocks of all bins of the round dealt out together
+      const int nblk = (liveLen + 31) >> 5;
+      {
+        int j = -1, base = 0, beg = 0, cnt = 0;   // bin j owns the items [base, base + cnt): its blocks beg, beg + 1, ...
+        for (int k = t;; k += NQ_LAB_THREADS) {
+          while (k >= base + cnt) {
+            if (++j == n) break;
+            base += cnt;
+            beg = (sFirstR[j] + 32) >> 5;
+            cnt = max(0, nblk - beg);
+          }
+          if (j == n) break;
+          const int blk = beg + (k - base);
+          if (!lab_block_skip(sProbe[j], V, blk, sErrR[j])) atomicOr(&sBits[j][blk >> 5], 1u << (blk & 31));
+        }
+      }
       __syncthreads();
-      if (w == 0) {                             // bit set -> ordered list
-        const unsigned m0 = sBits[2 * lane], m1 = sBits[2 * lane + 1];
-        const int c = __popc(m0) + __popc(m1);
+      for (int j = (int)w; j < n; j += W) {     // live blocks of each bin before each word of its bits
+        const int c0 = __popc(sBits[j][2 * lane]), c = c0 + __popc(sBits[j][2 * lane + 1]);
         int x = c;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= (unsigned)o) x += y; }
-        int at = x - c;
-        for (unsigned m = m0; m; m &= m - 1) sBlk[at++] = (unsigned short)(64 * lane + (__ffs(m) - 1));
-        for (unsigned m = m1; m; m &= m - 1) sBlk[at++] = (unsigned short)(64 * lane + 32 + (__ffs(m) - 1));
-        if (lane == 31) sNLive = x;
+        sPre[j][2 * lane] = (unsigned short)(x - c);
+        sPre[j][2 * lane + 1] = (unsigned short)(x - c + c0);
+        if (lane == 31) sPre[j][64] = (unsigned short)x;
       }
       __syncthreads();
       tick(2);
-      const int nLive = sNLive;
-      liveBlocks += nLive;
-      for (int g0 = 0; g0 < nLive; g0 += 32) {  // batches of 32 live blocks (<= 1024 bins), in list order
-        const int gn = min(32, nLive - g0);
-        // -- 3a. per-candidate lower bound (lab_cheap_keep): one warp per block, one lane per bin
-        if (t < 32) { sMaskA[t] = 0u; sMaskB[t] = 0u; }
+      // Batch g holds the live blocks 32 g .. 32 g + 31 of every bin of the round, bin-major: each bin is pruned and
+      // resolved on the schedule of a rescan of its own, and the round takes as many batches as its longest bin.
+      int nBatch = 0;
+      for (int j = 0; j < n; ++j) nBatch = max(nBatch, (sPre[j][64] + 31) >> 5);
+      for (int g = 0; g < nBatch; ++g) {
+        int gn = 0;                               // entries of this batch; thread t < gn makes entry t
+        {
+          int jt = -1, rt = 0;
+          for (int j = 0; j < n; ++j) {
+            const int e = min(32, max(0, (int)sPre[j][64] - 32 * g));
+            if (jt < 0 && t < gn + e) { jt = j; rt = 32 * g + t - gn; }
+            gn += e;
+          }
+          if (jt >= 0) {
+            int lo = 0, hi = 64;                  // the word of bin jt's rt-th live block
+            while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (sPre[jt][mid] <= rt) lo = mid; else hi = mid; }
+            const int blk = (lo << 5) + (int)__fns(sBits[jt][lo], 0, rt - sPre[jt][lo] + 1);
+            sBat[t] = (unsigned short)((jt << 11) | blk);
+          }
+        }
+        liveBlocks += gn;
+        // -- 3a. per-candidate lower bound (lab_cheap_keep): one warp per entry, one lane per bin
+        sMaskA[t] = 0u;
+        sMaskB[t] = 0u;
         __syncthreads();
-        for (int r0 = w; r0 < gn; r0 += 4 * W) {     // four records in flight per lane: the loads come from L2
+        for (int r0 = (int)w; r0 < gn; r0 += 4 * W) {     // four records in flight per lane: the loads come from L2
           float4 v[4];
+          int jr[4];
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int r = r0 + u * W;
-            const int i = r < gn ? ((int)sBlk[g0 + r] << 5) + (int)lane : -1;
-            v[u] = (i >= stop && i < liveLen) ? X.q[i] : make_float4(-1.f, 0.f, 0.f, 0.f);
+            const int e = r < gn ? (int)sBat[r] : 0;
+            jr[u] = e >> 11;
+            const int i = ((e & 2047) << 5) + (int)lane;
+            v[u] = (r < gn && i >= sFirstR[jr[u]] + 32 && i < liveLen) ? X.q[i] : dead;
           }
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int r = r0 + u * W;
-            const unsigned m = __ballot_sync(0xffffffffu, lab_cheap_keep_q(P, v[u], err));
+            const unsigned m = __ballot_sync(0xffffffffu, lab_cheap_keep_q(sProbe[jr[u]], v[u], sErrR[jr[u]]));
             if (lane == 0 && r < gn) sMaskA[r] = m;
           }
         }
         __syncthreads();
-        if (w == 0) {
-          const int c = __popc(sMaskA[lane]);
-          int x = c;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= (unsigned)o) x += y; }
-          sOffA[lane + 1] = x;
-          if (lane == 0) sOffA[0] = 0;
-        }
+        int totalA;
+        sOffA[t] = block_excl_scan_128(__popc(sMaskA[t]), &totalA, sScan);
+        if (t == 0) sOffA[NQ_LAB_THREADS] = totalA;
         __syncthreads();
-        const int totalA = sOffA[32];
-        // the s-th bin that passed 3a, in list order
-        auto posA = [&](int sIdx) {
-          int lo = 0, hi = 32;                    // largest r with sOffA[r] <= sIdx
+        // the s-th candidate that passed 3a, in batch order, and its bin of the round
+        auto posA = [&](int sIdx, int& j) {
+          int lo = 0, hi = gn;                    // largest r with sOffA[r] <= sIdx
           while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (sOffA[mid] <= sIdx) lo = mid; else hi = mid; }
-          return ((int)sBlk[g0 + lo] << 5) + (int)__fns(sMaskA[lo], 0, sIdx - sOffA[lo] + 1);
+          const int e = sBat[lo];
+          j = e >> 11;
+          return ((e & 2047) << 5) + (int)__fns(sMaskA[lo], 0, sIdx - sOffA[lo] + 1);
         };
-        // -- 3b. screen through the C' term, packed one bin per thread
+        // -- 3b. screen through the C' term, packed one candidate per thread
         for (int base = 0; base < totalA; base += NQ_LAB_THREADS) {
           const int sIdx = base + t;
-          LabCand dummy;
-          const bool keep = sIdx < totalA && lab_eval_t<true>(P, V, posA(sIdx), err, &dummy);
+          bool keep = false;
+          if (sIdx < totalA) {
+            int j;
+            const int i = posA(sIdx, j);
+            LabCand dummy;
+            keep = lab_eval_t<true>(sProbe[j], V, i, sErrR[j], &dummy);
+          }
           const unsigned m = __ballot_sync(0xffffffffu, keep);
           if (lane == 0) sMaskB[(base >> 5) + w] = m;
         }
         __syncthreads();
-        if (w == 0) {
-          const int c = __popc(sMaskB[lane]);
-          int x = c;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= (unsigned)o) x += y; }
-          sOffB[lane + 1] = x;
-          if (lane == 0) sOffB[0] = 0;
-        }
+        int total;
+        sOffB[t] = block_excl_scan_128(__popc(sMaskB[t]), &total, sScan);
         __syncthreads();
         tick(3);
-        const int total = sOffB[32];
         screened += total;
-        // -- 4. survivors in full, packed; then resolved in order
+        const int nW = (totalA + 31) >> 5;
+        // -- 4. survivors in full, packed; then each bin's resolved in its own list order against its own err
         for (int base = 0; base < total; base += NQ_LAB_THREADS) {
           const int uIdx = base + t;
-          int pos = -1;
+          int rec = 0;
           if (uIdx < total) {
-            int lo = 0, hi = 32;                  // largest word with sOffB[word] <= uIdx
+            int lo = 0, hi = nW;                  // largest word with sOffB[word] <= uIdx
             while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (sOffB[mid] <= uIdx) lo = mid; else hi = mid; }
             const int sIdx = (lo << 5) + (int)__fns(sMaskB[lo], 0, uIdx - sOffB[lo] + 1);   // index into the 3a list
-            const int i = posA(sIdx);
+            int j;
+            const int i = posA(sIdx, j);
             LabCand c;
-            if (lab_eval_t<false>(P, V, i, err, &c)) { pos = i; sGs[t] = c.gs; sGw[t] = c.gw; sF[t] = c.f; }
+            rec = j << 17;
+            if (lab_eval_t<false>(sProbe[j], V, i, sErrR[j], &c)) { rec |= (1 << 16) | i; sGs[t] = c.gs; sGw[t] = c.gw; sF[t] = c.f; }
           }
-          sPos[t] = pos;
+          sPos[t] = rec;
           fulls += uIdx < total;
           __syncthreads();
-          if (w == 0) {
+          if (w == 0) {                           // a bin's candidates are contiguous: the batch is bin-major
             const int cnt = min(NQ_LAB_THREADS, total - base);
             for (int q = 0; q < cnt; q += 32) {
               const int k = q + (int)lane;
+              const int rk = k < cnt ? sPos[k] : 0;
+              const bool alive = k < cnt && ((rk >> 16) & 1);
+              const int jk = k < cnt ? rk >> 17 : -1;
               LabCand c{0, 0, 0};
-              int pp = -1;
-              if (k < cnt) { pp = sPos[k]; if (pp >= 0) { c.gs = sGs[k]; c.gw = sGw[k]; c.f = sF[k]; } }
-              lab_accept_in_order(pp >= 0, c, pp, err, nn);
+              if (alive) { c.gs = sGs[k]; c.gw = sGw[k]; c.f = sF[k]; }
+              const int j0 = __shfl_sync(0xffffffffu, jk, 0), j1 = __shfl_sync(0xffffffffu, jk, min(31, cnt - 1 - q));
+              for (int j = j0; j <= j1; ++j) {
+                double err = sErrR[j];
+                int nn = sNnR[j];
+                lab_accept_in_order(alive && jk == j, c, rk & 0xFFFF, err, nn);
+                __syncwarp();
+                if (lane == 0) { sErrR[j] = err; sNnR[j] = nn; }
+              }
             }
-            if (lane == 0) { sErrCur = err; sNnCur = nn; }
           }
           __syncthreads();
           tick(4);
-          err = sErrCur; nn = sNnCur;
         }
       }
-      pairs += (unsigned long long)max(0, liveLen - first);
-      if (t == 0) {
-        // tb.tm = i; push slot down (PL:281-293)
-        float e1 = (float)err;
-        const int nnBin = nn < 0 ? 0 : live[nn];
-        S.bErr[b1] = e1; S.bNn[b1] = nnBin; S.bTm[b1] = sIter;
-        H.sift_down(pack_idnn(b1, nnBin), e1, sHeapN);
-      }
+      if (t < n) { const int nn = sNnR[t]; sNnR[t] = nn < 0 ? 0 : live[nn]; }
       __syncthreads();
-      tick(0);
       continue;
     }
 
     // ---- merge tb <- tb + nb (PL:297-311)
     if (t == 0) {
+      const int b1 = sB1;
       const int nbI = S.bNn[b1];
       const float n1 = S.bCnt[b1], n2 = S.bCnt[nbI];
       const float d = 1.0f / (n1 + n2);
@@ -830,10 +925,10 @@ __global__ void __launch_bounds__(NQ_LAB_THREADS, 4) k_merge_lab(NqImage* imgs, 
     I.statRescans = rescans; I.statPairs += pairs; I.statHeapPops = pops;
     for (int k = 0; k < 6; ++k) I.statCyc[k] = (unsigned long long)cyc[k];
     I.statLiveBlocks = liveBlocks; I.statScreened = screened;
+    I.statRounds = rounds; I.statDiscarded = discarded;
   }
   if (fulls) atomicAdd(&I.statFullEvals, fulls);
 }
-
 
 // -------------------------------------------------------------------------------------------------
 // RGB merge loop, same organisation as k_merge_lab: compacted records of the surviving bins, 32-bin
@@ -957,7 +1052,7 @@ __device__ __forceinline__ void rgb_accept_in_order(const RgbProbe& P, double ga
 
 static_assert(NQ_RGB_THREADS == NQ_LAB_THREADS, "block_excl_scan_128 is shared");
 
-__global__ void __launch_bounds__(NQ_RGB_THREADS, 4) k_merge_rgb(NqImage* imgs, const NqSlot* slots, int* liveBuf, int* posBuf, int logMerges, int rot) {
+__global__ void __launch_bounds__(NQ_RGB_THREADS, 4) k_merge_rgb(NqImage* imgs, const NqSlot* slots, int* liveBuf, int* posBuf, int logMerges) {
   extern __shared__ unsigned char smemRaw[];
   float* sErr = reinterpret_cast<float*>(smemRaw);
   unsigned* sId = reinterpret_cast<unsigned*>(smemRaw + (size_t)NQ_RGB_HEAP_SMEM * 4);
@@ -974,10 +1069,7 @@ __global__ void __launch_bounds__(NQ_RGB_THREADS, 4) k_merge_rgb(NqImage* imgs, 
   if (I.kind != NQ_KIND_RGB || I.nmax <= 2 || I.skipPnn) return;
   const NqSlot& S = slots[img];
   const RgbScratch X = rgb_scratch(S);
-  // The serial phases (heap top, ordered replay) belong to logical warp 0. Several CTAs share an SM, and the hardware
-  // places warp k of every CTA on the same scheduler: rotating the logical warp ids by the CTA index spreads the serial
-  // warps of co-resident images over the four schedulers.
-  const int t = (int)((threadIdx.x + 32u * (rot ? (blockIdx.x & 3u) : 0u)) & 127u);
+  const int t = threadIdx.x;
   const unsigned lane = lane_id(), w = t >> 5;
   const int W = NQ_RGB_THREADS / 32;
   const int maxbins = I.maxbins, extbins = I.extbins;

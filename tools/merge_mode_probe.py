@@ -4,7 +4,7 @@ hash of all palettes (the modes must agree bit for bit). The modes are the NQ_ME
 kept as profiles/r2_merge_variants.diff (not applied: the shipped library ignores the variable, every mode is the shipped
 kernel); NQ_AB_LIB=path loads another build of the library instead, for an old-vs-new comparison in one session.
 Usage: merge_mode_probe.py W H batch mode[,mode...]"""
-import hashlib, os, sys, time
+import ctypes, hashlib, os, sys, time
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import numpy as np
 import torch
@@ -12,6 +12,13 @@ from nquant_android_b200 import _lib
 if os.environ.get("NQ_AB_LIB"):          # an older build of the library, for an A/B in the same session
     _lib.SO = os.path.abspath(os.environ["NQ_AB_LIB"])
     _lib.SYMBOLS = []
+    if ctypes.CDLL(_lib.SO).nq_sizeof_image_info() != ctypes.sizeof(_lib.ImageInfo):   # built before the round counters
+
+        class _OldImageInfo(ctypes.Structure):
+            _fields_ = [f for f in _lib.ImageInfo._fields_ if f[0] not in ("merge_rounds", "rescans_discarded")]
+            as_dict = _lib.ImageInfo.as_dict
+
+        _lib.ImageInfo = _OldImageInfo
 from nquant_android_b200.quantizer import Context
 
 
@@ -48,7 +55,8 @@ def main():
         print(f"mode={mode:2d} {batch} x {W}x{H}: {dt:.3f} s {batch * npix / dt / 1e6:.1f} Mpix/s  merge={st['merge'][0]:.1f} ms  sweep={st['find_nn_sweep'][0]:.1f} ms  "
               f"palettes={hp} out0={ho} same_as_first={(hp, ho) == first}", flush=True)
         print("   merge Mcycles (image 0): " + "  ".join(f"{n}={c / 1e6:.0f}" for n, c in zip(names, mc)) +
-              f"  rescans={info['rescans']} full_evals={info['full_evals']} live_blocks={info['live_blocks']} screened={info['screened']}", flush=True)
+              f"  rescans={info['rescans']} rounds={info.get('merge_rounds', '-')} discarded={info.get('rescans_discarded', '-')} "
+              f"full_evals={info['full_evals']} live_blocks={info['live_blocks']} screened={info['screened']}", flush=True)
         ctx.close()
 
 
