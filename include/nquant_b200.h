@@ -152,6 +152,9 @@ typedef struct nq_image_info {
   /* CIELAB merge loop: rounds of rescans (stale heap entries rescanned together, see nq_pnn.cuh), and rescans computed
      in a round but not applied because a merge or the next round came first. `rescans` counts the applied ones only. */
   unsigned long long merge_rounds, rescans_discarded;
+  /* CTAs of the merge loop kernel of this image's kind (k_merge_lab or k_merge_rgb, one CTA per image) that one SM holds at
+     once, as the occupancy calculator reports it for this device */
+  int merge_ctas_per_sm;
 } nq_image_info;
 int nq_get_image_info(nq_ctx* ctx, int image, nq_image_info* out);
 /* sizeof(nq_image_info) as the library was built: lets a binding check its own mirror of the struct. */

@@ -37,6 +37,7 @@ class ImageInfo(ctypes.Structure):
         ("merge_cycles", ctypes.c_ulonglong * 6), ("live_blocks", ctypes.c_ulonglong), ("screened", ctypes.c_ulonglong),
         ("dither_cycles", ctypes.c_ulonglong * 3),
         ("merge_rounds", ctypes.c_ulonglong), ("rescans_discarded", ctypes.c_ulonglong),
+        ("merge_ctas_per_sm", ctypes.c_int),
     ]
 
     def as_dict(self):

@@ -180,6 +180,8 @@ struct nq_ctx {
   std::vector<cudaEvent_t> evPool;    // grows on demand, reused by every call
   size_t evUsed = 0;
   int smCount = 148;
+  // resident CTAs per SM of k_merge_lab<4>, k_merge_lab<8> and k_merge_rgb, from the occupancy calculator
+  int mergeLab4PerSm = 0, mergeLab8PerSm = 0, mergeRgbPerSm = 0;
   unsigned long long launches = 0;
   bool debug = false;
   int chunkImages = 0;                // images per chunk (0 = automatic)
@@ -386,6 +388,7 @@ struct NvtxRange {
 // One chunk of a call: images [base, base + n) of the group, with the events that bracket its stages.
 struct Chunk {
   int base = 0, n = 0;
+  int mergeInFlight = 0;           // images whose merge loops can run next to each other: this chunk's and a neighbour's
   cudaStream_t front = nullptr;
   int frontIdx = 0;
   cudaEvent_t evIn = nullptr;      // host-buffer calls: the chunk's pixels have arrived (copy-in stream)
@@ -549,6 +552,10 @@ struct GroupArgs {
   bool stopAfterSweep = false;   // stage hook nq_histogram: no merge loop, no dither
 };
 
+// Instance of k_merge_lab for a chunk: the one with 4 CTAs per SM has the shorter chain per image and is used while the merge
+// loops that can run at once (this chunk's and the other front stream's) fit one wave of it; beyond that, the one with 8.
+int lab_merge_ctas(const nq_ctx* c, const Chunk& ch) { return ch.mergeInFlight > c->smCount * c->mergeLab4PerSm ? 8 : 4; }
+
 // scan .. merge loop of one chunk, enqueued on its front stream (no host synchronisation unless the context is in debug mode)
 int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn, uint32_t* dOut) {
   NvtxRange nv("nq front (scan, histogram, find_nn, merge)");
@@ -564,6 +571,7 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
     I.kind = kind; I.width = A.w; I.height = A.h; I.npix = npix; I.nmax = nmax; I.dither = A.dither;
     I.seed = A.seeds ? A.seeds[ch.base + i] : 0ULL;
     I.transIdx = -1;
+    I.mergeCtas = kind == NQ_KIND_LAB ? (lab_merge_ctas(c, ch) == 8 ? c->mergeLab8PerSm : c->mergeLab4PerSm) : c->mergeRgbPerSm;
     NqSlot& S = c->hSlots[ch.base + i];
     S.in = dIn + (size_t)(ch.base + i) * npix;
     S.out = dOut + (size_t)(ch.base + i) * npix;
@@ -660,8 +668,10 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
     int* pos = c->dPos + (size_t)ch.base * NQ_NBINS;
     if (kind == NQ_KIND_RGB) {
       nq::k_merge_rgb<<<n, NQ_RGB_THREADS, (size_t)NQ_RGB_HEAP_SMEM * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0); ++c->launches;
+    } else if (lab_merge_ctas(c, ch) == 8) {
+      nq::k_merge_lab<8><<<n, NQ_LAB_THREADS, (size_t)nq::lab_heap_smem(8) * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0); ++c->launches;
     } else {
-      nq::k_merge_lab<<<n, NQ_LAB_THREADS, (size_t)NQ_LAB_HEAP_SMEM * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0); ++c->launches;
+      nq::k_merge_lab<4><<<n, NQ_LAB_THREADS, (size_t)nq::lab_heap_smem(4) * 8, st>>>(dI, dS, live, pos, c->debug ? 1 : 0); ++c->launches;
     }
   } else { mark(2); mark(3); }
   mark(4);
@@ -765,15 +775,18 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
   const uint32_t* dOrder = nullptr;
   int rc = ensure_order(c, A.w, A.h, &dOrder);
   if (rc) return rc;
-  // Chunk sizes. The merge loop wants >= 4 images per SM in flight, so chunks stay large: batches up to 640 images in one
-  // piece, larger ones in equal pieces of at most 512; host-buffer calls (from 32 images on) in at least two, so that the copies
-  // of one piece overlap the kernels of the other (a short first and last piece was tried and lost more in the merge loop than
-  // it hid). The device->host copy of a chunk starts while its dither is still running (SpecCudaBackend::done_prefix).
+  // Chunk sizes. The merge loop is the longest stage and its throughput grows with the images resident per SM, so a chunk
+  // holds as many images as the merge kernel's resident CTAs on the whole device (k_merge_lab<8> for CIELAB: 1184 on 148
+  // SMs, so a 1024-image batch runs all its merge loops in one wave, measured faster than two chunks of 512 on two front
+  // streams). Host-buffer calls (from 32 images on) go in at least two, so that the copies of one piece overlap the kernels
+  // of the other (a short first and last piece was tried and lost more in the merge loop than it hid). The device->host copy
+  // of a chunk starts while its dither is still running (SpecCudaBackend::done_prefix).
   std::vector<int> sizes;
   if (c->debug) sizes.push_back(n);
   else if (c->chunkImages > 0) { for (int b = 0; b < n; b += c->chunkImages) sizes.push_back(std::min(c->chunkImages, n - b)); }
   else {
-    const int pieces = std::max(n <= 640 ? 1 : (n + 511) / 512, (A.hIn && n >= 32) ? 2 : 1);
+    const int slots = c->smCount * (A.kind == NQ_KIND_LAB ? c->mergeLab8PerSm : c->mergeRgbPerSm);
+    const int pieces = std::max((n + slots - 1) / slots, (A.hIn && n >= 32) ? 2 : 1);
     for (int k = 0; k < pieces; ++k) sizes.push_back(n / pieces + (k < n % pieces ? 1 : 0));
   }
   const int nch = (int)sizes.size();
@@ -788,6 +801,7 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
   for (int k = 0, base = 0; k < nch; base += sizes[k], ++k) {
     Chunk& ch = chunks[k];
     ch.base = base; ch.n = sizes[k];
+    ch.mergeInFlight = sizes[k] + std::max(k > 0 ? sizes[k - 1] : 0, k + 1 < nch ? sizes[k + 1] : 0);   // two front streams
     ch.frontIdx = k % NQ_FRONT_STREAMS; ch.front = c->sFront[ch.frontIdx];
     for (auto& e : ch.ev) e = take_event(c);
     for (auto& e : ch.evD) e = take_event(c);
@@ -1017,7 +1031,12 @@ nq_ctx* nq_create(int device) {
   if (ok) ok = cudaFuncSetAttribute(nq::k_merge_rgb, cudaFuncAttributeMaxDynamicSharedMemorySize, NQ_RGB_HEAP_SMEM * 8) == cudaSuccess;
   if (ok) ok = cudaFuncSetAttribute(nq::k_hist_rgb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(nq::HistTable)) == cudaSuccess;
   if (ok) ok = cudaFuncSetAttribute(nq::k_dither_fifo, cudaFuncAttributeMaxDynamicSharedMemorySize, 32768) == cudaSuccess;
-  if (ok) ok = cudaFuncSetAttribute(nq::k_merge_lab, cudaFuncAttributeMaxDynamicSharedMemorySize, NQ_LAB_HEAP_SMEM * 8) == cudaSuccess;
+  if (ok) ok = cudaFuncSetAttribute(nq::k_merge_lab<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, nq::lab_heap_smem(4) * 8) == cudaSuccess &&
+               cudaFuncSetAttribute(nq::k_merge_lab<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, nq::lab_heap_smem(8) * 8) == cudaSuccess;
+  if (ok) ok = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->mergeLab4PerSm, nq::k_merge_lab<4>, NQ_LAB_THREADS, nq::lab_heap_smem(4) * 8) == cudaSuccess &&
+               cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->mergeLab8PerSm, nq::k_merge_lab<8>, NQ_LAB_THREADS, nq::lab_heap_smem(8) * 8) == cudaSuccess &&
+               cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->mergeRgbPerSm, nq::k_merge_rgb, NQ_RGB_THREADS, NQ_RGB_HEAP_SMEM * 8) == cudaSuccess &&
+               c->mergeLab4PerSm > 0 && c->mergeLab8PerSm > 0 && c->mergeRgbPerSm > 0;
   if (!ok) {
     fail(NQ_ERR_CUDA, std::string("context initialisation failed: ") + cudaGetErrorString(cudaGetLastError()));
     destroy_ctx(c, haveLut);          // drops the table reference taken above, the streams and every allocation
@@ -1164,6 +1183,7 @@ int nq_get_image_info(nq_ctx* c, int image, nq_image_info* o) {
   for (int k = 0; k < 6; ++k) o->merge_cycles[k] = I.statCyc[k];
   o->live_blocks = I.statLiveBlocks; o->screened = I.statScreened;
   o->merge_rounds = I.statRounds; o->rescans_discarded = I.statDiscarded;
+  o->merge_ctas_per_sm = I.mergeCtas;
   for (int k = 0; k < 3; ++k) o->dither_cycles[k] = I.statDither[k];
   o->error = I.error;
   return NQ_OK;

@@ -496,10 +496,15 @@ __device__ __forceinline__ unsigned pack_idnn(int id, int nn) { return (unsigned
 // pruned on the schedule of a rescan of its own. Thread 0 then replays the reference's top loop verbatim: a stale top with a result from the current
 // round takes it, one without starts the next round, and a merge discards the unused results. A wrong guess
 // costs work, never a different result.
-// 128 threads and 44 KB of heap per CTA: several images share an SM and fill each other's serial gaps.
+// 128 threads per CTA: several images share an SM and fill each other's serial gaps. The chain of one image is bound by
+// latency, so more images per SM buy throughput, and each image's chain gets longer as they share the SM. Two instances:
+// CTAS = 4 (128 registers, 44 KB of heap) has the shorter chain; CTAS = 8 (64 registers, a few spills at round boundaries,
+// 16 KB of heap, one more heap level in global memory) runs twice the images at once. The host launches the first when the
+// images in flight fit one wave of it and the second otherwise (lab_merge_ctas in nq_api.cu).
 // -------------------------------------------------------------------------------------------------
 #define NQ_LAB_THREADS 128
-#define NQ_LAB_HEAP_SMEM 5632   // 44 KB of heap: four CTAs fit one SM
+// heap slots kept in shared memory by the instance for `ctas` CTAs per SM (8 bytes each)
+__host__ __device__ constexpr int lab_heap_smem(int ctas) { return ctas >= 8 ? 2048 : 5632; }
 #define NQ_LAB_ROUND 4          // bins rescanned together in one round (8 would need 256-entry batches: more shared memory)
 
 __device__ __forceinline__ int block_excl_scan_128(int v, int* total, int* sScan /*[8]*/) {
@@ -551,12 +556,13 @@ __device__ __forceinline__ int rebuild_live_lab(const NqSlot& S, const LabScratc
   return total;
 }
 
-__global__ void __launch_bounds__(NQ_LAB_THREADS, 4) k_merge_lab(NqImage* imgs, const NqSlot* slots, int* liveBuf, int* posBuf, int logMerges) {
-  constexpr int R = NQ_LAB_ROUND;
+template <int CTAS>
+__global__ void __launch_bounds__(NQ_LAB_THREADS, CTAS) k_merge_lab(NqImage* imgs, const NqSlot* slots, int* liveBuf, int* posBuf, int logMerges) {
+  constexpr int R = NQ_LAB_ROUND, HS = lab_heap_smem(CTAS);
   static_assert(R >= 1 && 32 * R <= NQ_LAB_THREADS, "a batch holds 32 blocks of each bin of the round, one per thread");
   extern __shared__ unsigned char smemRaw[];
   float* sErr = reinterpret_cast<float*>(smemRaw);
-  unsigned* sId = reinterpret_cast<unsigned*>(smemRaw + (size_t)NQ_LAB_HEAP_SMEM * 4);
+  unsigned* sId = reinterpret_cast<unsigned*>(smemRaw + (size_t)HS * 4);
   __shared__ int sScan[8];
   __shared__ unsigned sBits[R][64];          // live blocks of each bin of the round, one bit per block
   __shared__ unsigned short sPre[R][65];     // live blocks of the bin before each word of sBits; [64]: all of them
@@ -584,7 +590,7 @@ __global__ void __launch_bounds__(NQ_LAB_THREADS, 4) k_merge_lab(NqImage* imgs, 
   const int maxbins = I.maxbins, extbins = I.extbins;
   int* live = liveBuf + (size_t)img * NQ_NBINS;
   int* posOf = posBuf + (size_t)img * NQ_NBINS;
-  HeapView<NQ_LAB_HEAP_SMEM> H{sErr, sId, S.heap};
+  HeapView<HS> H{sErr, sId, S.heap};
   const float4 dead = make_float4(-1.f, 0.f, 0.f, 0.f);
 
   // ---- heap build: sequential pushes in bin order (PL:246-257), replayed by warp 0

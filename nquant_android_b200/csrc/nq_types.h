@@ -43,6 +43,7 @@ struct NqImage {
   // merge-loop phase clocks (SM cycles, thread 0): 0 heap/top, 1 first-32, 2 block tests, 3 screen, 4 full+resolve, 5 merge+rebuild
   unsigned long long statCyc[6], statLiveBlocks, statScreened;
   unsigned long long statRounds, statDiscarded;   // CIELAB merge loop: rescan rounds, rescans computed but not applied
+  int mergeCtas;                                  // resident CTAs per SM of the merge loop instance launched (set by the host)
   unsigned long long statDither[3];   // FIFO dither: consumer cycles, consumer cycles waiting for the producer, producer cycles waiting
   int specDone;            // speculative segment-parallel dither (nq_dither_spec.cuh): 0 not its image, 1 dithered by it, 2 pending there,
                            // 3 handed back to k_dither_fifo

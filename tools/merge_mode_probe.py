@@ -12,10 +12,13 @@ from nquant_android_b200 import _lib
 if os.environ.get("NQ_AB_LIB"):          # an older build of the library, for an A/B in the same session
     _lib.SO = os.path.abspath(os.environ["NQ_AB_LIB"])
     _lib.SYMBOLS = []
-    if ctypes.CDLL(_lib.SO).nq_sizeof_image_info() != ctypes.sizeof(_lib.ImageInfo):   # built before the round counters
+    _old_size, _fields = ctypes.CDLL(_lib.SO).nq_sizeof_image_info(), list(_lib.ImageInfo._fields_)
+    while ctypes.sizeof(type("_I", (ctypes.Structure,), {"_fields_": _fields})) > _old_size:   # built before the last counters
+        _fields.pop()
+    if len(_fields) < len(_lib.ImageInfo._fields_):
 
         class _OldImageInfo(ctypes.Structure):
-            _fields_ = [f for f in _lib.ImageInfo._fields_ if f[0] not in ("merge_rounds", "rescans_discarded")]
+            _fields_ = _fields
             as_dict = _lib.ImageInfo.as_dict
 
         _lib.ImageInfo = _OldImageInfo
@@ -56,7 +59,8 @@ def main():
               f"palettes={hp} out0={ho} same_as_first={(hp, ho) == first}", flush=True)
         print("   merge Mcycles (image 0): " + "  ".join(f"{n}={c / 1e6:.0f}" for n, c in zip(names, mc)) +
               f"  rescans={info['rescans']} rounds={info.get('merge_rounds', '-')} discarded={info.get('rescans_discarded', '-')} "
-              f"full_evals={info['full_evals']} live_blocks={info['live_blocks']} screened={info['screened']}", flush=True)
+              f"full_evals={info['full_evals']} live_blocks={info['live_blocks']} screened={info['screened']} "
+              f"merge_ctas_per_sm={info.get('merge_ctas_per_sm', '-')}", flush=True)
         ctx.close()
 
 
