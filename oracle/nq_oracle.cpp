@@ -728,6 +728,7 @@ struct Trace {
   GilbertParams gp{};
   std::vector<float> gweights;
   int64_t rng_draws = 0, pixelMapSize = 0;
+  int64_t n_rescans = 0, n_heap_pops = 0;  // merge loop: find_nn calls on a stale top, deleted tops replaced by the last entry
   bool keep_draws = false;          // debugging aid of tests/spec_host_harness.cpp: the pixel (bidx) of every draw, in order
   std::vector<int32_t> draw_bidx;
   float bn_weight = 0;
@@ -892,10 +893,13 @@ class PnnQuantizer {
         int b1 = heap[1];
         tb = &bins[b1];
         if ((tb->tm >= tb->mtm) && (bins[tb->nn].mtm <= tb->tm)) break;
-        if (tb->mtm == 0xFFFF) b1 = heap[1] = heap[heap[0]--];
-        else {
+        if (tb->mtm == 0xFFFF) {
+          b1 = heap[1] = heap[heap[0]--];
+          ++trace.n_heap_pops;
+        } else {
           find_nn(bins, b1);
           tb->tm = i;
+          ++trace.n_rescans;
         }
         float err = bins[b1].err;
         for (l = 1; (l2 = l + l) <= heap[0]; l = l2) {
@@ -1305,10 +1309,13 @@ class PnnLABQuantizer : public PnnQuantizer {
         int b1 = heap[1];
         tb = &bins[b1];
         if ((tb->tm >= tb->mtm) && (bins[tb->nn].mtm <= tb->tm)) break;
-        if (tb->mtm == 0xFFFF) b1 = heap[1] = heap[heap[0]--];
-        else {
+        if (tb->mtm == 0xFFFF) {
+          b1 = heap[1] = heap[heap[0]--];
+          ++trace.n_heap_pops;
+        } else {
           find_nn(bins, b1, texicab);
           tb->tm = i;
+          ++trace.n_rescans;
         }
         float err = bins[b1].err;
         for (l = 1; (l2 = l + l) <= heap[0]; l = l2) {
@@ -1564,6 +1571,7 @@ struct nqo_scalars {
   float beta, bn_weight;
   double weight, weight_final, ratio_init, ratio_merge, PR, PG, PB, PA, gweight;
   long long rng_draws, pixelMapSize, n_merges, n_saliencies, n_gweights, n_bins, n_init;
+  long long n_rescans, n_heap_pops;
 };
 void nqo_get_scalars(nqo_handle* h, nqo_scalars* s) {
   const Trace& t = h->trace;
@@ -1577,6 +1585,7 @@ void nqo_get_scalars(nqo_handle* h, nqo_scalars* s) {
   s->rng_draws = t.rng_draws; s->pixelMapSize = t.pixelMapSize; s->n_merges = (long long)t.merges.size() / 2;
   s->n_saliencies = (long long)t.saliencies.size(); s->n_gweights = (long long)t.gweights.size();
   s->n_bins = (long long)t.bins.size() / 5; s->n_init = (long long)t.init_err.size();
+  s->n_rescans = t.n_rescans; s->n_heap_pops = t.n_heap_pops;
 }
 void nqo_get_bins(nqo_handle* h, double* bins5) { memcpy(bins5, h->trace.bins.data(), h->trace.bins.size() * 8); }
 void nqo_get_init_nn(nqo_handle* h, float* err, int* nn) {

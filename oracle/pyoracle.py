@@ -25,7 +25,8 @@ class Scalars(ctypes.Structure):
                  "transparentColor", "margin", "thresold", "DITHER_MAX", "ditherMax", "sortedByYDiff", "hasAlpha"]] + \
                [("beta", ctypes.c_float), ("bn_weight", ctypes.c_float)] + \
                [(n, ctypes.c_double) for n in ["weight", "weight_final", "ratio_init", "ratio_merge", "PR", "PG", "PB", "PA", "gweight"]] + \
-               [(n, ctypes.c_longlong) for n in ["rng_draws", "pixelMapSize", "n_merges", "n_saliencies", "n_gweights", "n_bins", "n_init"]]
+               [(n, ctypes.c_longlong) for n in ["rng_draws", "pixelMapSize", "n_merges", "n_saliencies", "n_gweights", "n_bins", "n_init",
+                                                    "n_rescans", "n_heap_pops"]]
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}
