@@ -107,6 +107,29 @@ int nq_convert_batch_device(nq_ctx* ctx, int kind, const uint32_t* d_argb_in, in
                             int n_max_colors, int dither, const uint64_t* rng_seeds, uint32_t* d_argb_out,
                             uint32_t* palettes_out, int* palette_lens, int* has_alpha);
 
+/* A batch of images of DIFFERENT sizes in HOST memory: image i is widths[i] x heights[i] pixels at argb_in[i], its result
+ * goes to argb_out[i] (the reference's "one quantizer per file" loop, MainActivity.java:190-194, as one call). kind,
+ * n_max_colors and dither apply to every image; rng_seeds, palettes_out (256 entries per image), palette_lens and has_alpha
+ * as in nq_convert_batch. Each image gets exactly what nq_convert gives it alone; nq_get_image_info(ctx, i, ..) and the
+ * debug getters address image i of the call. Every side must be 1..65535. The images share one pass through the
+ * pipeline, so a folder of mixed sizes keeps the GPU as full as a batch of one size does; the workspace is laid out for
+ * the largest image of the call (see DESIGN.md section 3). */
+int nq_convert_ragged(nq_ctx* ctx, int kind, const uint32_t* const* argb_in, const int* widths, const int* heights,
+                      int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds, uint32_t* const* argb_out,
+                      uint32_t* palettes_out, int* palette_lens, int* has_alpha);
+
+/* The same with DEVICE buffers on the context's GPU: the images packed back to back (image i starts at pixel
+ * sum_{j<i} widths[j]*heights[j]), base pointers 16-byte aligned, e.g. torch.cat of the flattened images. */
+int nq_convert_ragged_device(nq_ctx* ctx, int kind, const uint32_t* d_argb_in, const int* widths, const int* heights,
+                             int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds, uint32_t* d_argb_out,
+                             uint32_t* palettes_out, int* palette_lens, int* has_alpha);
+
+/* nq_convert_ragged over several contexts with the dynamic queue of nq_convert_batch_multi (pieces of queue_images
+ * images, 0 = one piece per context). */
+int nq_convert_ragged_multi(nq_ctx** contexts, int n_contexts, int kind, const uint32_t* const* argb_in, const int* widths,
+                            const int* heights, int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds,
+                            uint32_t* const* argb_out, uint32_t* palettes_out, int* palette_lens, int* has_alpha, int queue_images);
+
 /* Stage hook (parity + profiling): GilbertCurve.dither / BlueNoise.dither with a caller-supplied
  * palette (PnnQuantizer.java:393-407, PnnLABQuantizer.java:492-522). Runs the alpha scan and the
  * histogram-derived scalars as convert() would, but replaces the palette pnnquan produced by
@@ -124,7 +147,8 @@ int nq_histogram(nq_ctx* ctx, int kind, const uint32_t* argb_in, int width, int 
                  double* bins5, float* init_err, int* init_nn, int capacity);
 
 /* Generalized Hilbert visiting order for a width x height image (GilbertCurve.java:282-334,
- * 356-365): order_out[n] = x + y*width of the n-th pixel diffusePixel is called on. Host buffer. */
+ * 356-365): order_out[n] = x + y*width of the n-th pixel diffusePixel is called on. Host buffer. Computed on the host
+ * by the same position -> pixel function (csrc/nq_gilbert.h) that builds the convert calls' tables on the device. */
 int nq_gilbert_order(int width, int height, uint32_t* order_out);
 
 /* ---- introspection of the last batch (parity tests, bench counters) --------------------------- */

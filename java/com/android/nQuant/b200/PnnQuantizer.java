@@ -132,6 +132,57 @@ public class PnnQuantizer implements AutoCloseable {
 		}
 	}
 
+	/**
+	 * The same for images of DIFFERENT sizes (a folder of photos as it comes): image i is widths[i] x heights[i] pixels.
+	 * One call over every image (nq_convert_ragged_multi), so images of all sizes share the pipeline instead of one call per
+	 * size; each image gets exactly what convert() gives it alone. Sides must be 1..65535. Like the rest of this package,
+	 * written against the C ABI and not compiled here (no JDK in the build image).
+	 */
+	public static int[][] convertBatch(boolean lab, int[][] images, int[] widths, int[] heights, int nMaxColors, boolean dither,
+	                                   long[] rngSeeds, int[] devices, int[][] palettesOut) throws Exception {
+		final int n = images.length;
+		if (widths.length != n || heights.length != n)
+			throw new IllegalArgumentException("one width and one height per image");
+		try (Arena arena = Arena.ofConfined()) {
+			MemorySegment ins = arena.allocate(ValueLayout.ADDRESS, n);
+			MemorySegment outs = arena.allocate(ValueLayout.ADDRESS, n);
+			MemorySegment[] out = new MemorySegment[n];
+			for (int i = 0; i < n; ++i) {
+				final long npix = (long) widths[i] * heights[i];
+				if (images[i].length != npix)
+					throw new IllegalArgumentException("image " + i + " does not hold widths[i]*heights[i] pixels");
+				ins.setAtIndex(ValueLayout.ADDRESS, i, arena.allocateFrom(ValueLayout.JAVA_INT, images[i]));
+				out[i] = arena.allocate(ValueLayout.JAVA_INT, npix);
+				outs.setAtIndex(ValueLayout.ADDRESS, i, out[i]);
+			}
+			MemorySegment w = arena.allocateFrom(ValueLayout.JAVA_INT, widths);
+			MemorySegment h = arena.allocateFrom(ValueLayout.JAVA_INT, heights);
+			MemorySegment pal = arena.allocate(ValueLayout.JAVA_INT, 256L * n);
+			MemorySegment plen = arena.allocate(ValueLayout.JAVA_INT, n);
+			MemorySegment seeds = rngSeeds == null ? MemorySegment.NULL : arena.allocateFrom(ValueLayout.JAVA_LONG, rngSeeds);
+			MemorySegment ctxs = arena.allocate(ValueLayout.ADDRESS, devices.length);
+			for (int g = 0; g < devices.length; ++g)
+				ctxs.setAtIndex(ValueLayout.ADDRESS, g, NQuantNative.context(devices[g]));
+			int rc;
+			try {
+				rc = (int) NQuantNative.nq_convert_ragged_multi.invokeExact(ctxs, devices.length,
+					lab ? NQuantNative.NQ_KIND_PNNLAB : NQuantNative.NQ_KIND_PNN, ins, w, h, n, nMaxColors, dither ? 1 : 0,
+					seeds, outs, pal, plen, MemorySegment.NULL, 0);
+			} catch (Throwable t) {
+				throw new Exception(t);
+			}
+			if (rc != 0)
+				throw new Exception("nq_convert_ragged_multi failed (" + rc + "): " + NQuantNative.lastError());
+			int[][] res = new int[n][];
+			for (int i = 0; i < n; ++i) {
+				res[i] = out[i].toArray(ValueLayout.JAVA_INT);
+				if (palettesOut != null)
+					palettesOut[i] = pal.asSlice(4L * 256 * i, 4L * plen.getAtIndex(ValueLayout.JAVA_INT, i)).toArray(ValueLayout.JAVA_INT);
+			}
+			return res;
+		}
+	}
+
 	/** Quantizer objects share their thread's context (NQuantNative.context); nothing to release per object. */
 	@Override
 	public void close() {

@@ -13,6 +13,7 @@ SYMBOLS = [
     "nq_debug_get_bins", "nq_debug_get_merges", "nq_debug_get_saliencies", "nq_kernel_launches", "nq_debug_math",
     "nq_synth_device", "nq_get_stage_times", "nq_set_stream", "nq_debug_ciede", "nq_sizeof_image_info",
     "nq_set_spec_dither", "nq_get_spec_stats", "nq_reset_stream", "nq_set_chunk_images", "nq_get_kernel_times", "nq_convert_batch_multi", "nq_histogram",
+    "nq_convert_ragged", "nq_convert_ragged_device", "nq_convert_ragged_multi",
 ]
 
 NQ_KIND_PNN, NQ_KIND_PNNLAB = 0, 1
@@ -66,6 +67,9 @@ def load():
     L.nq_convert_batch.argtypes = [vp, ci, vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp]
     L.nq_convert_batch_device.argtypes = [vp, ci, vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp]
     L.nq_convert_batch_multi.argtypes = [vp, ci, ci, vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp, ci]
+    L.nq_convert_ragged.argtypes = [vp, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp]
+    L.nq_convert_ragged_device.argtypes = [vp, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp]
+    L.nq_convert_ragged_multi.argtypes = [vp, ci, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, ci]
     L.nq_dither_with_palette.argtypes = [vp, ci, vp, ci, ci, ci, ci, u64, vp, ci, vp]
     L.nq_gilbert_order.argtypes = [ci, ci, vp]
     L.nq_histogram.argtypes = [vp, ci, vp, ci, ci, ci, vp, vp, vp, vp, ci]

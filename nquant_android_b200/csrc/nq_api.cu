@@ -24,6 +24,7 @@
 #include "nq_pnn.cuh"
 #include "nq_dither.cuh"
 #include "nq_dither_spec.cuh"
+#include "nq_gilbert.h"
 
 #define NQ_NSTAGES 6   // scan, histogram, find_nn sweep, merge, dither setup + saliency, dither
 #define NQ_NKERNELS 4  // kernels timed on their own (nq_get_kernel_times): 0 k_spec_run, 1 k_dither_fifo, 2 k_dither_sorted, 3 k_merge_*
@@ -45,36 +46,18 @@ int fail(int code, const std::string& msg) {
 
 const signed char kBlueNoise[4096] = NQ_BLUE_NOISE_INIT;
 
-// ---- generalized Hilbert order (GC:282-334, 356-365), explicit stack -----------------------------
-struct GFrame { int x, y, ax, ay, bx, by; };
-inline int sgn(int v) { return (v > 0) - (v < 0); }
-template <class Emit>
-void gilbert_walk(int width, int height, Emit emit) {
-  std::vector<GFrame> st;
-  st.reserve(256);
-  if (width >= height) st.push_back({0, 0, width, 0, 0, height});
-  else st.push_back({0, 0, 0, height, width, 0});
-  while (!st.empty()) {
-    GFrame f = st.back();
-    st.pop_back();
-    int x = f.x, y = f.y;
-    const int ax = f.ax, ay = f.ay, bx = f.bx, by = f.by;
-    const int w = abs(ax + ay), h = abs(bx + by);
-    const int dax = sgn(ax), day = sgn(ay), dbx = sgn(bx), dby = sgn(by);
-    if (h == 1) { for (int i = 0; i < w; ++i) { emit(x, y); x += dax; y += day; } continue; }
-    if (w == 1) { for (int i = 0; i < h; ++i) { emit(x, y); x += dbx; y += dby; } continue; }
-    int ax2 = ax / 2, ay2 = ay / 2, bx2 = bx / 2, by2 = by / 2;
-    const int w2 = abs(ax2 + ay2), h2 = abs(bx2 + by2);
-    if (2 * w > 3 * h) {
-      if ((w2 % 2) != 0 && w > 2) { ax2 += dax; ay2 += day; }
-      st.push_back({x + ax2, y + ay2, ax - ax2, ay - ay2, bx, by});   // visited second
-      st.push_back({x, y, ax2, ay2, bx, by});                          // visited first
-      continue;
+// ---- generalized Hilbert order (GC:282-334, 356-365): the tables of every size a call needs, one launch ----------
+struct GilbertJob { int w, h; uint32_t* dst; };
+// one thread per curve position; blockIdx.y strides over the tables
+__global__ void k_gilbert_order(const GilbertJob* jobs, int njobs) {
+  for (int j = blockIdx.y; j < njobs; j += gridDim.y) {
+    const GilbertJob J = jobs[j];
+    const unsigned long long npix = (unsigned long long)J.w * (unsigned long long)J.h;
+    for (unsigned long long n = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; n < npix; n += (unsigned long long)gridDim.x * blockDim.x) {
+      int x, y;
+      nq::gilbert_xy(J.w, J.h, n, &x, &y);
+      J.dst[n] = (uint32_t)x | ((uint32_t)y << 16);
     }
-    if ((h2 % 2) != 0 && h > 2) { bx2 += dbx; by2 += dby; }
-    st.push_back({x + (ax - dax) + (bx2 - dbx), y + (ay - day) + (by2 - dby), -bx2, -by2, -(ax - ax2), -(ay - ay2)});
-    st.push_back({x + bx2, y + by2, ax, ay, bx - bx2, by - by2});
-    st.push_back({x, y, bx2, by2, ax2, ay2});
   }
 }
 
@@ -185,10 +168,12 @@ struct nq_ctx {
   unsigned long long launches = 0;
   bool debug = false;
   int chunkImages = 0;                // images per chunk (0 = automatic)
-  // Gilbert orders by (w,h), least recently used first in orderLru
+  // Gilbert orders by (w,h), least recently used first in orderLru; dJobs: the size list of k_gilbert_order
   std::map<std::pair<int, int>, uint32_t*> orders;
   std::vector<std::pair<int, int>> orderLru;
   size_t orderBytes = 0;
+  GilbertJob* dJobs = nullptr;
+  int jobsCap = 0;
   // workspace
   unsigned char* ws = nullptr;
   size_t wsBytes = 0;
@@ -283,7 +268,8 @@ int ensure_workspace(nq_ctx* c, int kind, int npix, int wantSlots, bool needBits
   if (NQ_FRONT_STREAMS * pool * sortSet + perImage > budget) return fail(NQ_ERR_NOMEM, "not enough device memory for one image workspace");
   const int maxSlots = (int)std::min<size_t>((budget - NQ_FRONT_STREAMS * pool * sortSet) / perImage, 8192);
   const int slots = std::min(wantSlots, maxSlots);
-  if (c->ws && c->wsKind == kind && c->wsNpix == npix && c->wsSlots >= slots && c->wsDebug == c->debug && c->wsBits == needBits && c->wsIdx == needIdx) return NQ_OK;
+  // a workspace built for larger images serves smaller ones (slots are laid out by the largest image of the call)
+  if (c->ws && c->wsKind == kind && c->wsNpix >= npix && c->wsSlots >= slots && c->wsDebug == c->debug && c->wsBits == needBits && c->wsIdx == needIdx) return NQ_OK;
   if (c->ws) { CU(cudaDeviceSynchronize()); cudaFree(c->ws); c->ws = nullptr; c->wsBytes = 0; c->wsSlots = 0; }
   const size_t imgsB = align_up(sizeof(NqImage) * slots, 256), slotsB = align_up(sizeof(NqSlot) * slots, 256);
   const size_t liveB = align_up((size_t)slots * NQ_NBINS * 4, 256);
@@ -327,41 +313,72 @@ int ensure_workspace(nq_ctx* c, int kind, int npix, int wantSlots, bool needBits
   return NQ_OK;
 }
 
-// The visiting order of a (w, h) image is a table of 4 bytes per pixel, built by a host walk the first time the size is
-// seen. The cache is bounded (entries and bytes): a long-lived context that serves many sizes evicts the least recently used.
+// The visiting order of a (w, h) image is a table of 4 bytes per pixel (x | y << 16), built on the device the first time the
+// size is seen: one k_gilbert_order launch for every new size of a call, on the dither stream (the only streams that read the
+// tables are that one and the aux stream forked from it). The cache is bounded (entries and bytes): a long-lived context
+// that serves many sizes evicts the least recently used. The sizes of the running call are never evicted, so a call with
+// many sizes may take the cache past its bound; the bound applies again at the next call. Called before anything of the
+// call is enqueued. order[i]: the table of image i.
 #define NQ_ORDER_MAX_ENTRIES 8
 #define NQ_ORDER_MAX_BYTES ((size_t)2 << 30)
-int ensure_order(nq_ctx* c, int w, int h, const uint32_t** out) {
-  auto key = std::make_pair(w, h);
-  auto it = c->orders.find(key);
-  if (it != c->orders.end()) {
+int ensure_orders(nq_ctx* c, int n, const int* ws, const int* hs, std::vector<const uint32_t*>& order) {
+  typedef std::pair<int, int> Size;
+  std::map<Size, int> used;                         // sizes of this call
+  std::vector<Size> missing;
+  size_t addBytes = 0;
+  for (int i = 0; i < n; ++i) {
+    const Size key(ws[i], hs[i]);
+    if (!used.emplace(key, 0).second) continue;
     auto pos = std::find(c->orderLru.begin(), c->orderLru.end(), key);
-    if (pos != c->orderLru.end()) { c->orderLru.erase(pos); c->orderLru.push_back(key); }
-    *out = it->second;
-    return NQ_OK;
+    if (pos != c->orderLru.end()) { c->orderLru.erase(pos); c->orderLru.push_back(key); }   // most recently used
+    else { missing.push_back(key); addBytes += (size_t)key.first * key.second * 4; }
   }
-  if (w > 65535 || h > 65535) return fail(NQ_ERR_ARG, "image side exceeds 65535");
-  const size_t bytes = (size_t)w * h * 4;
-  while (!c->orderLru.empty() && (c->orderLru.size() >= NQ_ORDER_MAX_ENTRIES || c->orderBytes + bytes > NQ_ORDER_MAX_BYTES)) {
-    const auto old = c->orderLru.front();
-    c->orderLru.erase(c->orderLru.begin());
-    CU(cudaDeviceSynchronize());                    // nothing in flight may still read the table
-    cudaFree(c->orders[old]);
-    c->orderBytes -= (size_t)old.first * old.second * 4;
-    c->orders.erase(old);
+  bool synced = false;
+  for (auto it = c->orderLru.begin(); it != c->orderLru.end() && !used.count(*it) &&
+       (c->orderLru.size() + missing.size() > NQ_ORDER_MAX_ENTRIES || c->orderBytes + addBytes > NQ_ORDER_MAX_BYTES);) {
+    if (!synced) { CU(cudaDeviceSynchronize()); synced = true; }   // nothing in flight may still read the table
+    cudaFree(c->orders[*it]);
+    c->orderBytes -= (size_t)it->first * it->second * 4;
+    c->orders.erase(*it);
+    it = c->orderLru.erase(it);
   }
-  std::vector<uint32_t> host;
-  host.reserve((size_t)w * h);
-  gilbert_walk(w, h, [&](int x, int y) { host.push_back((uint32_t)x | ((uint32_t)y << 16)); });
-  if (host.size() != (size_t)w * h) return fail(NQ_ERR_ARG, "gilbert walk size mismatch");
-  uint32_t* d = nullptr;
-  CU(cudaMalloc(&d, bytes));
-  cudaError_t e = cudaMemcpy(d, host.data(), bytes, cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) { cudaFree(d); return fail(NQ_ERR_CUDA, std::string("cudaMemcpy(order): ") + cudaGetErrorString(e)); }
-  c->orders[key] = d;
-  c->orderLru.push_back(key);
-  c->orderBytes += bytes;
-  *out = d;
+  if (!missing.empty()) {
+    std::vector<GilbertJob> jobs;
+    unsigned long long maxNpix = 0;
+    cudaError_t e = cudaSuccess;
+    for (const Size& key : missing) {
+      uint32_t* d = nullptr;
+      const size_t bytes = (size_t)key.first * key.second * 4;
+      e = cudaMalloc(&d, bytes);
+      if (e != cudaSuccess) break;
+      jobs.push_back({key.first, key.second, d});
+      maxNpix = std::max<unsigned long long>(maxNpix, bytes / 4);
+    }
+    if (e == cudaSuccess && c->jobsCap < (int)jobs.size()) {
+      if (c->dJobs) cudaFree(c->dJobs);                  // (synchronises: the previous call's launch has read it)
+      c->dJobs = nullptr; c->jobsCap = 0;
+      e = cudaMalloc(&c->dJobs, sizeof(GilbertJob) * jobs.size());
+      if (e == cudaSuccess) c->jobsCap = (int)jobs.size();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(c->dJobs, jobs.data(), sizeof(GilbertJob) * jobs.size(), cudaMemcpyHostToDevice, c->sDith);
+    if (e == cudaSuccess) {
+      const int gx = (int)std::min<unsigned long long>((maxNpix + 255) / 256, (unsigned long long)c->smCount * 16);
+      k_gilbert_order<<<dim3(gx, std::min<int>((int)jobs.size(), 65535)), 256, 0, c->sDith>>>(c->dJobs, (int)jobs.size()); ++c->launches;
+      e = cudaGetLastError();
+    }
+    if (e != cudaSuccess) {                              // no table that was not built stays in the cache
+      for (const GilbertJob& j : jobs) cudaFree(j.dst);
+      return fail(e == cudaErrorMemoryAllocation ? NQ_ERR_NOMEM : NQ_ERR_CUDA, std::string("Gilbert order tables: ") + cudaGetErrorString(e));
+    }
+    for (const GilbertJob& j : jobs) {
+      const Size key(j.w, j.h);
+      c->orders[key] = j.dst;
+      c->orderLru.push_back(key);
+      c->orderBytes += (size_t)j.w * j.h * 4;
+    }
+  }
+  order.resize(n);
+  for (int i = 0; i < n; ++i) order[i] = c->orders[Size(ws[i], hs[i])];
   return NQ_OK;
 }
 
@@ -385,6 +402,47 @@ struct NvtxRange {
   ~NvtxRange() { nvtxRangePop(); }
 };
 
+// Images [0, n) of a group, every one with its own geometry; the per-image pointers start at the group's first image.
+// Pixels are packed back to back in the call's device buffers: image i at dIn + off[i], off[i + 1] - off[i] pixels.
+struct GroupArgs {
+  int kind, nmax, dither;
+  const int* w;
+  const int* h;
+  const size_t* off;                // n + 1 entries
+  const uint32_t* const* order;     // Gilbert table of each image's size (nullptr with stopAfterSweep)
+  const uint64_t* seeds;
+  const uint32_t* dPalIn;
+  int palInLen;
+  const uint32_t* const* hIn;       // host pixels of each image (nullptr: dIn is the caller's device buffer and already holds them)
+  uint32_t* const* hOut;
+  bool stopAfterSweep = false;      // stage hook nq_histogram: no merge loop, no dither
+};
+
+int max_npix(const GroupArgs& A, int base, int n) {
+  int m = 1;
+  for (int i = base; i < base + n; ++i) m = std::max(m, A.w[i] * A.h[i]);
+  return m;
+}
+
+// Copies of images [from, to) between the packed device buffer and the caller's host pointers: one copy per run of images
+// that are contiguous in host memory as well (an equal-size batch from one array is one copy).
+cudaError_t copy_in(const GroupArgs& A, int from, int to, uint32_t* dIn, cudaStream_t st) {
+  for (int i = from, j; i < to; i = j) {
+    for (j = i + 1; j < to && A.hIn[j] == A.hIn[i] + (A.off[j] - A.off[i]); ++j) {}
+    cudaError_t e = cudaMemcpyAsync(dIn + A.off[i], A.hIn[i], (A.off[j] - A.off[i]) * 4, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
+cudaError_t copy_out(const GroupArgs& A, int from, int to, const uint32_t* dOut, cudaStream_t st) {
+  for (int i = from, j; i < to; i = j) {
+    for (j = i + 1; j < to && A.hOut[j] == A.hOut[i] + (A.off[j] - A.off[i]); ++j) {}
+    cudaError_t e = cudaMemcpyAsync(A.hOut[i], dOut + A.off[i], (A.off[j] - A.off[i]) * 4, cudaMemcpyDeviceToHost, st);
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
+
 // One chunk of a call: images [base, base + n) of the group, with the events that bracket its stages.
 struct Chunk {
   int base = 0, n = 0;
@@ -399,9 +457,8 @@ struct Chunk {
   unsigned long long launches[NQ_NSTAGES] = {};
   // host-buffer calls: images [0, copied) of the chunk are already on their way to the host (progressive copy-out)
   int copied = 0;
-  uint32_t* hOut = nullptr;        // host destination of the chunk's first image, or nullptr
-  const uint32_t* dOut = nullptr;  // device source of the chunk's first image
-  size_t imageBytes = 0;
+  const GroupArgs* A = nullptr;    // the group's host destinations (GroupArgs::hOut), or nullptr
+  const uint32_t* dOut = nullptr;  // the call's packed device output
 };
 
 // launches and small copies of the admission / round loop (spec_drive in nq_dither_spec.cuh) on the dither stream
@@ -447,12 +504,11 @@ struct SpecCudaBackend {
   }
   // images [0, prefix) of the chunk are complete: copy them out on the copy-out stream while the rest is still being dithered
   void done_prefix(int prefix) {
-    if (!ch->hOut || prefix - ch->copied < 16) return;
+    if (!ch->A || prefix - ch->copied < 16) return;
     cudaEvent_t e = take_event(c);
     keep(cudaEventRecord(e, st));
     keep(cudaStreamWaitEvent(c->sOut, e, 0));
-    keep(cudaMemcpyAsync(ch->hOut + (size_t)ch->copied * (ch->imageBytes / 4), ch->dOut + (size_t)ch->copied * (ch->imageBytes / 4),
-                         (size_t)(prefix - ch->copied) * ch->imageBytes, cudaMemcpyDeviceToHost, c->sOut));
+    keep(copy_out(*ch->A, ch->base + ch->copied, ch->base + prefix, ch->dOut, c->sOut));
     ch->copied = prefix;
   }
   void note(int round, int active, int open, int patches, int redos) {
@@ -464,17 +520,18 @@ struct SpecCudaBackend {
 // serial kernels of the other images can be enqueued in between. spec_prepare: the pool of work-array slots and
 // k_spec_setup, which decides on the device which images are taken (NqImage::specDone = 2, elig[i] = 1) -- synchronises.
 // spec_rounds: the admission / round loop; images it completes get specDone = 1, images it took but could not finish 3
-// (listed in `handed`).
-struct SpecPlan { int seg = 0, nslots = 0, any = 0; };
-int spec_prepare(nq_ctx* c, Chunk& ch, cudaStream_t st, int npix, const uint32_t* dOrder, std::vector<int>& elig, SpecPlan* plan) {
+// (listed in `handed`). The pool's slots and the launch grids are sized by the chunk's largest image; every kernel of the
+// path bounds its loops by its own image.
+struct SpecPlan { int seg = 0, nslots = 0, any = 0, npix = 0; };
+int spec_prepare(nq_ctx* c, Chunk& ch, cudaStream_t st, const GroupArgs& A, std::vector<int>& elig, SpecPlan* plan) {
   using namespace nq::spec;
-  const int n = ch.n;
+  const int n = ch.n, npix = max_npix(A, ch.base, n);
   elig.assign(n, 0);
   *plan = SpecPlan{};
   int seg = c->specSeg;
   const int warm = c->specWarm;
   if (seg == 0) {   // automatic: 8192-pixel segments when that gives the machine enough threads, shorter ones for small jobs
-    const long long total = (long long)n * (long long)npix;
+    const long long total = (long long)(A.off[ch.base + n] - A.off[ch.base]);
     seg = total / 8192 >= 32768 ? 8192 : (int)std::max<long long>(2048, (total / 32768 + 255) / 256 * 256);
     if (seg > 8192) seg = 8192;
   }
@@ -516,14 +573,14 @@ int spec_prepare(nq_ctx* c, Chunk& ch, cudaStream_t st, int npix, const uint32_t
   spec_bind_pool(pool.data(), nslots, c->specBuf, L);
   CU(cudaMemcpyAsync(c->dSpecPool, pool.data(), sizeof(SpecWork) * (size_t)nslots, cudaMemcpyHostToDevice, st));
   int* dElig = reinterpret_cast<int*>(c->specBuf);      // scratch: the pool's work arrays are not in use yet
-  k_spec_setup<<<(n + 63) / 64, 64, 0, st>>>(c->dImgs + ch.base, c->dSlots + ch.base, c->dSpec + ch.base, dOrder, n, seg, warm, dElig); ++c->launches;
+  k_spec_setup<<<(n + 63) / 64, 64, 0, st>>>(c->dImgs + ch.base, c->dSlots + ch.base, c->dSpec + ch.base, nullptr, n, seg, warm, dElig); ++c->launches;
   CU(cudaMemcpyAsync(elig.data(), dElig, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));                    // also keeps `pool` alive until the copy is done
   for (int i = 0; i < n; ++i) plan->any += (elig[i] & 255) == 1;
-  plan->seg = seg; plan->nslots = nslots;
+  plan->seg = seg; plan->nslots = nslots; plan->npix = npix;
   return NQ_OK;
 }
-int spec_rounds(nq_ctx* c, Chunk& ch, cudaStream_t st, int npix, const SpecPlan& plan, const std::vector<int>& elig, std::vector<int>& handed) {
+int spec_rounds(nq_ctx* c, Chunk& ch, cudaStream_t st, const SpecPlan& plan, const std::vector<int>& elig, std::vector<int>& handed) {
   using namespace nq::spec;
   handed.clear();
   if (!plan.any) return NQ_OK;
@@ -532,7 +589,7 @@ int spec_rounds(nq_ctx* c, Chunk& ch, cudaStream_t st, int npix, const SpecPlan&
   be.begin();
   SpecStats stats;
   handed.assign(plan.any, 0);
-  spec_drive(be, c->dImgs + ch.base, c->dSpec + ch.base, c->dSpecPool, elig.data(), ch.n, npix, plan.seg, plan.nslots, c->dSpecInts, c->dTanh,
+  spec_drive(be, c->dImgs + ch.base, c->dSpec + ch.base, c->dSpecPool, elig.data(), ch.n, plan.npix, plan.seg, plan.nslots, c->dSpecInts, c->dTanh,
              c->smCount, &stats, handed.data());
   handed.resize((size_t)stats.handedBack);
   be.end();
@@ -542,16 +599,6 @@ int spec_rounds(nq_ctx* c, Chunk& ch, cudaStream_t st, int npix, const SpecPlan&
   return NQ_OK;
 }
 
-struct GroupArgs {
-  int kind, w, h, nmax, dither;
-  const uint64_t* seeds;
-  const uint32_t* dPalIn;
-  int palInLen;
-  const uint32_t* hIn;     // host pixels (nullptr: dIn is the caller's device buffer and already holds them)
-  uint32_t* hOut;
-  bool stopAfterSweep = false;   // stage hook nq_histogram: no merge loop, no dither
-};
-
 // Instance of k_merge_lab for a chunk: the one with 4 CTAs per SM has the shorter chain per image and is used while the merge
 // loops that can run at once (this chunk's and the other front stream's) fit one wave of it; beyond that, the one with 8.
 int lab_merge_ctas(const nq_ctx* c, const Chunk& ch) { return ch.mergeInFlight > c->smCount * c->mergeLab4PerSm ? 8 : 4; }
@@ -559,7 +606,7 @@ int lab_merge_ctas(const nq_ctx* c, const Chunk& ch) { return ch.mergeInFlight >
 // scan .. merge loop of one chunk, enqueued on its front stream (no host synchronisation unless the context is in debug mode)
 int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn, uint32_t* dOut) {
   NvtxRange nv("nq front (scan, histogram, find_nn, merge)");
-  const int n = ch.n, npix = A.w * A.h, kind = A.kind, nmax = A.nmax;
+  const int n = ch.n, kind = A.kind, nmax = A.nmax;
   cudaStream_t st = ch.front;
   NqImage* dI = c->dImgs + ch.base;
   NqSlot* dS = c->dSlots + ch.base;
@@ -568,13 +615,15 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
   for (int i = 0; i < n; ++i) {
     NqImage& I = hImgs[i];
     memset(&I, 0, sizeof(I));
-    I.kind = kind; I.width = A.w; I.height = A.h; I.npix = npix; I.nmax = nmax; I.dither = A.dither;
-    I.seed = A.seeds ? A.seeds[ch.base + i] : 0ULL;
+    const int g = ch.base + i;
+    I.kind = kind; I.width = A.w[g]; I.height = A.h[g]; I.npix = A.w[g] * A.h[g]; I.nmax = nmax; I.dither = A.dither;
+    I.seed = A.seeds ? A.seeds[g] : 0ULL;
     I.transIdx = -1;
     I.mergeCtas = kind == NQ_KIND_LAB ? (lab_merge_ctas(c, ch) == 8 ? c->mergeLab8PerSm : c->mergeLab4PerSm) : c->mergeRgbPerSm;
-    NqSlot& S = c->hSlots[ch.base + i];
-    S.in = dIn + (size_t)(ch.base + i) * npix;
-    S.out = dOut + (size_t)(ch.base + i) * npix;
+    NqSlot& S = c->hSlots[g];
+    S.in = dIn + A.off[g];
+    S.out = dOut + A.off[g];
+    S.order = A.order ? A.order[g] : nullptr;
     if (kind == NQ_KIND_LAB) {   // sort scratch: the sets of this chunk's front stream, cycled through the chunk
       unsigned char* sp = c->sortPool + c->sortSetBytes * ((size_t)ch.frontIdx * c->sortSets + (size_t)(i % c->sortSets));
       S.sortA = reinterpret_cast<uint32_t*>(sp);
@@ -587,6 +636,8 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
   CU(cudaMemsetAsync(c->zeroPlane + c->zeroSlotBytes * ch.base, 0, c->zeroSlotBytes * n, st));
   CU(cudaMemsetAsync(c->memoPlane + c->memoSlotBytes * ch.base, 0xFF, c->memoSlotBytes * n, st));
   for (int i = 0; i < n; ++i) if (c->hSlots[ch.base + i].bits) CU(cudaMemsetAsync(c->hSlots[ch.base + i].bits, 0, (size_t)1 << 29, st));
+  // grids of the per-pixel kernels come from the chunk's largest image; the kernels bound their loops by their own image
+  const int npix = max_npix(A, ch.base, n);
   const int gx = pixel_grid_x(c, npix, n);
   const dim3 pg(gx, n);
   unsigned long long l0 = c->launches;
@@ -598,7 +649,8 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
   if (nmax > 2) {
     if (kind == NQ_KIND_RGB) {
       {  // contiguous tiles per CTA; enough CTAs to fill the machine twice over
-        const int ntiles = ((A.w + NQ_HTW - 1) / NQ_HTW) * ((A.h + NQ_HTW - 1) / NQ_HTW);
+        int ntiles = 1;
+        for (int g = ch.base; g < ch.base + n; ++g) ntiles = std::max(ntiles, ((A.w[g] + NQ_HTW - 1) / NQ_HTW) * ((A.h[g] + NQ_HTW - 1) / NQ_HTW));
         const dim3 hg(std::max(1, std::min(ntiles, std::max(1, c->smCount * 8 / n))), n);
         nq::k_hist_rgb<<<hg, 256, sizeof(nq::HistTable), st>>>(dI, dS); ++c->launches;
       }
@@ -681,9 +733,9 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
 
 // dither of one chunk on the dither stream (after its front). The speculative path's rounds synchronise with the host;
 // the serial kernels of the images it does not take run next to it on the aux stream.
-int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dOrder) {
+int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A) {
   NvtxRange nv("nq dither (setup, Gilbert pass, BlueNoise pass)");
-  const int n = ch.n, npix = A.w * A.h, kind = A.kind;
+  const int n = ch.n, npix = max_npix(A, ch.base, n), kind = A.kind;
   cudaStream_t st = c->sDith, ax = c->sAux;
   NqImage* dI = c->dImgs + ch.base;
   NqSlot* dS = c->dSlots + ch.base;
@@ -704,7 +756,7 @@ int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dOrder)
   const bool spec = c->specDither && kind == NQ_KIND_LAB && A.dither;
   SpecPlan plan;
   if (spec) {
-    int rc = spec_prepare(c, ch, st, npix, dOrder, elig, &plan);
+    int rc = spec_prepare(c, ch, st, A, elig, &plan);
     if (rc) return rc;
   }
   // Everything the speculative path did not take (specDone == 0) goes through the serial kernels on the aux stream, next
@@ -715,11 +767,11 @@ int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dOrder)
   CU(cudaStreamWaitEvent(ax, evFork, 0));
   ch.evK[2] = take_event(c); ch.evK[3] = take_event(c);
   cudaEventRecord(ch.evK[2], ax);
-  nq::k_dither_fifo<<<n, 64, cacheBytes, ax>>>(dI, dS, dOrder, cacheBytes, 0); ++c->launches;
+  nq::k_dither_fifo<<<n, 64, cacheBytes, ax>>>(dI, dS, cacheBytes, 0); ++c->launches;
   cudaEventRecord(ch.evK[3], ax);
   ch.evK[4] = take_event(c); ch.evK[5] = take_event(c);
   cudaEventRecord(ch.evK[4], ax);
-  nq::k_dither_sorted<<<n, 32, 0, ax>>>(dI, dS, dOrder); ++c->launches;
+  nq::k_dither_sorted<<<n, 32, 0, ax>>>(dI, dS); ++c->launches;
   cudaEventRecord(ch.evK[5], ax);
   if (kind == NQ_KIND_RGB && !A.dither && A.nmax > 32) {   // BlueNoise.dither second pass, one thread per pixel (images flagged bnParallel)
     nq::k_bn_rgb_init<<<dim3(8, n), 256, 0, ax>>>(dI, dS); ++c->launches;
@@ -728,13 +780,13 @@ int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dOrder)
     nq::k_bn_rgb_c<<<pg, 256, 0, ax>>>(dI, dS); ++c->launches;
   }
   if (spec) {
-    int rc = spec_rounds(c, ch, st, npix, plan, elig, handed);
+    int rc = spec_rounds(c, ch, st, plan, elig, handed);
     if (rc) return rc;
     if (!handed.empty()) {   // qualifying images the rounds gave up on (specDone == 3): the serial kernel after all
       cudaEvent_t evBack = take_event(c);
       CU(cudaEventRecord(evBack, st));
       CU(cudaStreamWaitEvent(ax, evBack, 0));
-      nq::k_dither_fifo<<<n, 64, cacheBytes, ax>>>(dI, dS, dOrder, cacheBytes, 3); ++c->launches;
+      nq::k_dither_fifo<<<n, 64, cacheBytes, ax>>>(dI, dS, cacheBytes, 3); ++c->launches;
     }
   }
   CU(cudaEventRecord(evJoin, ax));
@@ -745,14 +797,33 @@ int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dOrder)
   return NQ_OK;
 }
 
+int check_size(int w, int h) {
+  if (w <= 0 || h <= 0) return fail(NQ_ERR_ARG, "n_images, width and height must be positive");
+  if (w > 65535 || h > 65535) return fail(NQ_ERR_ARG, "image side exceeds 65535");   // the order tables pack x | y << 16
+  if ((long long)w * h > 0x7fffffffLL / 4) return fail(NQ_ERR_ARG, "image too large");
+  return NQ_OK;
+}
 int check_args(nq_ctx* c, int kind, const void* in, int n, int w, int h, int nmax, const void* out) {
   if (!c) return fail(NQ_ERR_ARG, "null context");
   if (kind != NQ_KIND_PNN && kind != NQ_KIND_PNNLAB) return fail(NQ_ERR_ARG, "kind must be NQ_KIND_PNN or NQ_KIND_PNNLAB");
   if (!in || !out) return fail(NQ_ERR_ARG, "null pixel buffer");
-  if (n <= 0 || w <= 0 || h <= 0) return fail(NQ_ERR_ARG, "n_images, width and height must be positive");
-  if ((long long)w * h > 0x7fffffffLL / 4) return fail(NQ_ERR_ARG, "image too large");
+  if (n <= 0) return fail(NQ_ERR_ARG, "n_images, width and height must be positive");
+  int rc = check_size(w, h);
+  if (rc) return rc;
   if (nmax < 2) return fail(NQ_ERR_ARG, "n_max_colors must be >= 2 (the reference indexes palette[1], PnnQuantizer.java:446)");
   if (nmax > NQ_MAXK) return fail(NQ_ERR_UNSUPPORTED, "n_max_colors > 256 is not supported by this build");
+  return NQ_OK;
+}
+// a ragged call: the arrays of sides (and, for host buffers, of per-image pointers) are checked before any work starts
+int check_ragged(nq_ctx* c, int kind, const void* in, const int* ws, const int* hs, int n, int nmax, const void* out,
+                 const uint32_t* const* hIn = nullptr, uint32_t* const* hOut = nullptr) {
+  int rc = check_args(c, kind, in, n, 1, 1, nmax, out);
+  if (rc) return rc;
+  if (!ws || !hs) return fail(NQ_ERR_ARG, "null widths or heights");
+  for (int i = 0; i < n; ++i) {
+    if ((rc = check_size(ws[i], hs[i]))) return fail(rc, "image " + std::to_string(i) + ": " + g_lastError);
+    if ((hIn && !hIn[i]) || (hOut && !hOut[i])) return fail(NQ_ERR_ARG, "image " + std::to_string(i) + ": null pixel buffer");
+  }
   return NQ_OK;
 }
 
@@ -769,12 +840,10 @@ int collect_results(nq_ctx* c, int base, int n, uint32_t* palettes, int* plens, 
 
 // convert() for images [0, n) of a group that fits the workspace: the group is cut into chunks that flow through
 // front streams (scan .. merge), the dither stream and the copy-out stream, so that one chunk's merge loop, the previous
-// chunk's dither and the host copies of both overlap. dIn / dOut are device buffers holding (or receiving, A.hIn) the pixels.
+// chunk's dither and the host copies of both overlap. dIn / dOut are the call's packed device buffers holding (or receiving,
+// A.hIn) the pixels, image i of the group at A.off[i].
 int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uint32_t* dOut, int dbgBase) {
-  const int npix = A.w * A.h;
-  const uint32_t* dOrder = nullptr;
-  int rc = ensure_order(c, A.w, A.h, &dOrder);
-  if (rc) return rc;
+  int rc = NQ_OK;
   // Chunk sizes. The merge loop is the longest stage and its throughput grows with the images resident per SM, so a chunk
   // holds as many images as the merge kernel's resident CTAs on the whole device (k_merge_lab<8> for CIELAB: 1184 on 148
   // SMs, so a 1024-image batch runs all its merge loops in one wave, measured faster than two chunks of 512 on two front
@@ -807,7 +876,7 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
     for (auto& e : ch.evD) e = take_event(c);
     if (A.hIn) {   // every chunk's pixels are copied in on their own stream, in order, as early as the copy engine allows
       ch.evIn = take_event(c);
-      CU(cudaMemcpyAsync(const_cast<uint32_t*>(dIn) + (size_t)ch.base * npix, A.hIn + (size_t)ch.base * npix, (size_t)ch.n * npix * 4, cudaMemcpyHostToDevice, c->sIn));
+      CU(copy_in(A, ch.base, ch.base + ch.n, const_cast<uint32_t*>(dIn), c->sIn));
       CU(cudaEventRecord(ch.evIn, c->sIn));
     }
   }
@@ -822,14 +891,13 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
       for (auto& e : chunks[k].evD) CU(cudaEventRecord(e, c->sDith));
       continue;
     }
-    if (A.hOut) { chunks[k].hOut = A.hOut + (size_t)chunks[k].base * npix; chunks[k].dOut = dOut + (size_t)chunks[k].base * npix; chunks[k].imageBytes = (size_t)npix * 4; }
-    rc = run_dither(c, chunks[k], G, dOrder);
+    if (A.hOut) { chunks[k].A = &G; chunks[k].dOut = dOut; }
+    rc = run_dither(c, chunks[k], G);
     if (rc) return rc;
     if (A.hOut && chunks[k].copied < chunks[k].n) {   // device -> host of what the progressive copy-out has not taken yet
       Chunk& ch = chunks[k];
       CU(cudaStreamWaitEvent(c->sOut, ch.evD[2], 0));
-      CU(cudaMemcpyAsync(A.hOut + (size_t)(ch.base + ch.copied) * npix, dOut + (size_t)(ch.base + ch.copied) * npix, (size_t)(ch.n - ch.copied) * npix * 4,
-                         cudaMemcpyDeviceToHost, c->sOut));
+      CU(copy_out(A, ch.base + ch.copied, ch.base + ch.n, dOut, c->sOut));
     }
   }
   CU(cudaEventRecord(evOut, c->sOut));
@@ -864,35 +932,40 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
       D.merges.assign((size_t)merges * 2, 0);
       if (merges && c->hSlots[i].mergeLog) CU(cudaMemcpy(D.merges.data(), c->hSlots[i].mergeLog, (size_t)merges * 8, cudaMemcpyDeviceToHost));
       D.sal.clear();
-      if (I.gUseSal && c->hSlots[i].sal) { D.sal.resize(npix); CU(cudaMemcpy(D.sal.data(), c->hSlots[i].sal, (size_t)npix * 4, cudaMemcpyDeviceToHost)); }
+      if (I.gUseSal && c->hSlots[i].sal) { D.sal.resize(I.npix); CU(cudaMemcpy(D.sal.data(), c->hSlots[i].sal, (size_t)I.npix * 4, cudaMemcpyDeviceToHost)); }
     }
   }
   return NQ_OK;
 }
 
-// dIn / dOut: device buffers for the whole batch. hIn / hOut (optional): host buffers the batch is read from / written to
-// chunk by chunk, overlapped with the kernels.
-int convert_device(nq_ctx* c, int kind, const uint32_t* dIn, int n, int w, int h, int nmax, int dither, const uint64_t* seeds,
-                   uint32_t* dOut, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn, int palInLen,
-                   const uint32_t* hIn = nullptr, uint32_t* hOut = nullptr, bool stopAfterSweep = false) {
+// Every convert entry point, equal sizes or not, ends here. Image i is ws[i] x hs[i] pixels; dIn / dOut: device buffers of
+// the whole call, the images packed back to back. hIn / hOut (optional): one host pointer per image, read from / written to
+// chunk by chunk, overlapped with the kernels. The workspace is sized by the largest image of the call.
+int convert_device(nq_ctx* c, int kind, int n, const int* ws, const int* hs, const uint32_t* dIn, uint32_t* dOut, int nmax, int dither,
+                   const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn, int palInLen,
+                   const uint32_t* const* hIn = nullptr, uint32_t* const* hOut = nullptr, bool stopAfterSweep = false) {
   CU(cudaSetDevice(c->device));
-  const int npix = w * h;
+  std::vector<size_t> off(n + 1, 0);
+  int npix = 1;
+  for (int i = 0; i < n; ++i) { off[i + 1] = off[i] + (size_t)ws[i] * hs[i]; npix = std::max(npix, ws[i] * hs[i]); }
   // the BlueNoise second pass of PnnLABQuantizer weighs by pixelMap.size() (PL:511-513): track it only then
   const bool needBits = kind == NQ_KIND_LAB && !dither && nmax > 32;
   // PnnQuantizer's BlueNoise second pass runs one thread per pixel and keeps the first-pass indices next to the output
   const bool needIdx = kind == NQ_KIND_RGB && !dither && nmax > 32;
   int rc = ensure_workspace(c, kind, npix, n, needBits, needIdx);
   if (rc) return rc;
+  std::vector<const uint32_t*> order;
+  if (!stopAfterSweep && (rc = ensure_orders(c, n, ws, hs, order))) return rc;
   if (c->debug) c->dbg.assign(n, DebugImage{});
   int firstErr = 0;
   std::vector<NqImage> all;
   all.reserve(n);
   for (int base = 0; base < n; base += c->wsSlots) {
     const int m = std::min(c->wsSlots, n - base);
-    GroupArgs A{kind, w, h, nmax, dither, seeds ? seeds + base : nullptr, dPalIn, palInLen,
-                hIn ? hIn + (size_t)base * npix : nullptr, hOut ? hOut + (size_t)base * npix : nullptr};
+    GroupArgs A{kind, nmax, dither, ws + base, hs + base, off.data() + base, order.empty() ? nullptr : order.data() + base,
+                seeds ? seeds + base : nullptr, dPalIn, palInLen, hIn ? hIn + base : nullptr, hOut ? hOut + base : nullptr};
     A.stopAfterSweep = stopAfterSweep;
-    rc = convert_group(c, A, m, dIn + (size_t)base * npix, dOut + (size_t)base * npix, base);
+    rc = convert_group(c, A, m, dIn, dOut, base);
     if (rc) return rc;
     collect_results(c, base, m, palettes, plens, hasAlpha, &firstErr);
     all.insert(all.end(), c->lastImgs.begin(), c->lastImgs.end());
@@ -917,6 +990,35 @@ int ensure_stage(nq_ctx* c, size_t bytes) {
   return NQ_OK;
 }
 
+// host-buffer calls: the images go through the context's staging buffers (sized by the call's total pixels)
+int convert_host(nq_ctx* c, int kind, int n, const int* ws, const int* hs, const uint32_t* const* in, uint32_t* const* out, int nmax,
+                 int dither, const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn = nullptr,
+                 int palInLen = 0, bool stopAfterSweep = false) {
+  CU(cudaSetDevice(c->device));
+  size_t total = 0;
+  for (int i = 0; i < n; ++i) total += (size_t)ws[i] * hs[i];
+  int rc = ensure_stage(c, total * 4);
+  if (rc) return rc;
+  rc = convert_device(c, kind, n, ws, hs, c->dIn, c->dOut, nmax, dither, seeds, palettes, plens, hasAlpha, dPalIn, palInLen, in, out, stopAfterSweep);
+  if (rc) return rc;
+  CU(cudaStreamSynchronize(c->stream));
+  return NQ_OK;
+}
+
+// An equal-size batch as the per-image arrays of the ragged path: image i at base + i * w * h.
+struct UniformBatch {
+  std::vector<int> w, h;
+  std::vector<const uint32_t*> in;
+  std::vector<uint32_t*> out;
+  UniformBatch(int n, int width, int height, const uint32_t* hIn = nullptr, uint32_t* hOut = nullptr) : w(n, width), h(n, height) {
+    const size_t npix = (size_t)width * height;
+    if (hIn) for (int i = 0; i < n; ++i) in.push_back(hIn + i * npix);
+    if (hOut) for (int i = 0; i < n; ++i) out.push_back(hOut + i * npix);
+  }
+  const uint32_t* const* ins() const { return in.empty() ? nullptr : in.data(); }
+  uint32_t* const* outs() { return out.empty() ? nullptr : out.data(); }
+};
+
 }  // namespace
 
 namespace {
@@ -929,6 +1031,7 @@ void destroy_ctx(nq_ctx* c, bool dropLut) {
     if (it != g_lut.end() && it->second.refs > 0 && --it->second.refs == 0) { cudaFree(it->second.ptr); g_lut.erase(it); }
   }
   for (auto& kv : c->orders) cudaFree(kv.second);
+  if (c->dJobs) cudaFree(c->dJobs);
   if (c->ws) cudaFree(c->ws);
   if (c->dIn) cudaFree(c->dIn);
   if (c->dOut) cudaFree(c->dOut);
@@ -962,6 +1065,44 @@ __global__ void k_spec_tables(float* tanhTab, float* w3) {
     nq::init_weights(w, DM);
     for (int k = 0; k < NQ_MAXQ + 3; ++k) w3[t * (NQ_MAXQ + 3) + k] = k < DM ? w[k] : 0.f;
   }
+}
+}  // namespace
+
+namespace {
+// One worker thread per context pulls pieces of the batch from a shared counter (a dynamic queue: a GPU that finishes early
+// takes the next piece) and runs convert(context, first image, images) on its piece. No collective: the images are independent.
+template <class Convert>
+int run_multi(nq_ctx** ctxs, int nctx, int n, int queueImages, Convert convert) {
+  const int piece = queueImages > 0 ? queueImages : (n + nctx - 1) / nctx;   // default: one piece per context
+  std::atomic<int> next(0), firstRc(NQ_OK);
+  std::mutex errMutex;
+  std::string errMsg;
+  auto worker = [&](int g) {
+    for (;;) {
+      const int base = next.fetch_add(piece);
+      if (base >= n || firstRc.load() != NQ_OK) return;
+      const int m = std::min(piece, n - base);
+      const int r = convert(ctxs[g], base, m);
+      if (r != NQ_OK) {
+        std::lock_guard<std::mutex> lk(errMutex);
+        int expected = NQ_OK;
+        if (firstRc.compare_exchange_strong(expected, r)) errMsg = "context " + std::to_string(g) + ", images " + std::to_string(base) + ".." + std::to_string(base + m - 1) + ": " + nq_last_error();
+        return;
+      }
+    }
+  };
+  std::vector<std::thread> threads;
+  for (int g = 1; g < nctx; ++g) threads.emplace_back(worker, g);
+  worker(0);
+  for (auto& t : threads) t.join();
+  if (firstRc.load() != NQ_OK) return fail(firstRc.load(), errMsg);
+  return NQ_OK;
+}
+int check_contexts(nq_ctx** ctxs, int nctx, int queueImages) {
+  if (!ctxs || nctx <= 0) return fail(NQ_ERR_ARG, "no contexts");
+  for (int g = 0; g < nctx; ++g) if (!ctxs[g]) return fail(NQ_ERR_ARG, "null context in the list");
+  if (queueImages < 0) return fail(NQ_ERR_ARG, "queue_images must be >= 0");
+  return NQ_OK;
 }
 }  // namespace
 
@@ -1055,7 +1196,16 @@ int nq_convert_batch_device(nq_ctx* c, int kind, const uint32_t* d_in, int n, in
   int rc = check_args(c, kind, d_in, n, w, h, nmax, d_out);
   if (rc) return rc;
   NvtxRange nv("nq_convert_batch_device");
-  return convert_device(c, kind, d_in, n, w, h, nmax, dither, seeds, d_out, palettes, plens, hasAlpha, nullptr, 0);
+  UniformBatch B(n, w, h);
+  return convert_device(c, kind, n, B.w.data(), B.h.data(), d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0);
+}
+
+int nq_convert_ragged_device(nq_ctx* c, int kind, const uint32_t* d_in, const int* ws, const int* hs, int n, int nmax, int dither,
+                             const uint64_t* seeds, uint32_t* d_out, uint32_t* palettes, int* plens, int* hasAlpha) {
+  int rc = check_ragged(c, kind, d_in, ws, hs, n, nmax, d_out);
+  if (rc) return rc;
+  NvtxRange nv("nq_convert_ragged_device");
+  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0);
 }
 
 int nq_convert_batch(nq_ctx* c, int kind, const uint32_t* in, int n, int w, int h, int nmax, int dither, const uint64_t* seeds,
@@ -1063,53 +1213,43 @@ int nq_convert_batch(nq_ctx* c, int kind, const uint32_t* in, int n, int w, int 
   int rc = check_args(c, kind, in, n, w, h, nmax, out);
   if (rc) return rc;
   NvtxRange nv("nq_convert_batch");
-  CU(cudaSetDevice(c->device));
-  const size_t bytes = (size_t)n * w * h * 4;
-  rc = ensure_stage(c, bytes);
-  if (rc) return rc;
   // host -> device, kernels and device -> host are interleaved chunk by chunk inside convert_device
-  rc = convert_device(c, kind, c->dIn, n, w, h, nmax, dither, seeds, c->dOut, palettes, plens, hasAlpha, nullptr, 0, in, out);
-  if (rc) return rc;
-  CU(cudaStreamSynchronize(c->stream));
-  return NQ_OK;
+  UniformBatch B(n, w, h, in, out);
+  return convert_host(c, kind, n, B.w.data(), B.h.data(), B.ins(), B.outs(), nmax, dither, seeds, palettes, plens, hasAlpha);
 }
 
-// One worker thread per context pulls pieces of the batch from a shared counter (a dynamic queue: a GPU that finishes early
-// takes the next piece) and runs nq_convert_batch on its piece. No collective: the images are independent.
+int nq_convert_ragged(nq_ctx* c, int kind, const uint32_t* const* in, const int* ws, const int* hs, int n, int nmax, int dither,
+                      const uint64_t* seeds, uint32_t* const* out, uint32_t* palettes, int* plens, int* hasAlpha) {
+  int rc = check_ragged(c, kind, in, ws, hs, n, nmax, out, in, out);
+  if (rc) return rc;
+  NvtxRange nv("nq_convert_ragged");
+  return convert_host(c, kind, n, ws, hs, in, out, nmax, dither, seeds, palettes, plens, hasAlpha);
+}
+
 int nq_convert_batch_multi(nq_ctx** ctxs, int nctx, int kind, const uint32_t* in, int n, int w, int h, int nmax, int dither,
                            const uint64_t* seeds, uint32_t* out, uint32_t* palettes, int* plens, int* hasAlpha, int queueImages) {
-  if (!ctxs || nctx <= 0) return fail(NQ_ERR_ARG, "no contexts");
-  for (int g = 0; g < nctx; ++g) if (!ctxs[g]) return fail(NQ_ERR_ARG, "null context in the list");
-  int rc = check_args(ctxs[0], kind, in, n, w, h, nmax, out);
+  int rc = check_contexts(ctxs, nctx, queueImages);
   if (rc) return rc;
-  if (queueImages < 0) return fail(NQ_ERR_ARG, "queue_images must be >= 0");
-  const int piece = queueImages > 0 ? queueImages : (n + nctx - 1) / nctx;   // default: one piece per context
+  if ((rc = check_args(ctxs[0], kind, in, n, w, h, nmax, out))) return rc;
   const size_t npix = (size_t)w * h;
-  std::atomic<int> next(0), firstRc(NQ_OK);
-  std::mutex errMutex;
-  std::string errMsg;
-  auto worker = [&](int g) {
-    for (;;) {
-      const int base = next.fetch_add(piece);
-      if (base >= n || firstRc.load() != NQ_OK) return;
-      const int m = std::min(piece, n - base);
-      const int r = nq_convert_batch(ctxs[g], kind, in + (size_t)base * npix, m, w, h, nmax, dither, seeds ? seeds + base : nullptr,
-                                     out + (size_t)base * npix, palettes ? palettes + (size_t)base * NQ_MAXK : nullptr,
-                                     plens ? plens + base : nullptr, hasAlpha ? hasAlpha + base : nullptr);
-      if (r != NQ_OK) {
-        std::lock_guard<std::mutex> lk(errMutex);
-        int expected = NQ_OK;
-        if (firstRc.compare_exchange_strong(expected, r)) errMsg = "context " + std::to_string(g) + ", images " + std::to_string(base) + ".." + std::to_string(base + m - 1) + ": " + nq_last_error();
-        return;
-      }
-    }
-  };
-  std::vector<std::thread> threads;
-  for (int g = 1; g < nctx; ++g) threads.emplace_back(worker, g);
-  worker(0);
-  for (auto& t : threads) t.join();
-  if (firstRc.load() != NQ_OK) return fail(firstRc.load(), errMsg);
-  return NQ_OK;
+  return run_multi(ctxs, nctx, n, queueImages, [&](nq_ctx* c, int base, int m) {
+    return nq_convert_batch(c, kind, in + (size_t)base * npix, m, w, h, nmax, dither, seeds ? seeds + base : nullptr,
+                            out + (size_t)base * npix, palettes ? palettes + (size_t)base * NQ_MAXK : nullptr,
+                            plens ? plens + base : nullptr, hasAlpha ? hasAlpha + base : nullptr);
+  });
+}
+
+int nq_convert_ragged_multi(nq_ctx** ctxs, int nctx, int kind, const uint32_t* const* in, const int* ws, const int* hs, int n, int nmax,
+                            int dither, const uint64_t* seeds, uint32_t* const* out, uint32_t* palettes, int* plens, int* hasAlpha,
+                            int queueImages) {
+  int rc = check_contexts(ctxs, nctx, queueImages);
+  if (rc) return rc;
+  if ((rc = check_ragged(ctxs[0], kind, in, ws, hs, n, nmax, out, in, out))) return rc;
+  return run_multi(ctxs, nctx, n, queueImages, [&](nq_ctx* c, int base, int m) {
+    return nq_convert_ragged(c, kind, in + base, ws + base, hs + base, m, nmax, dither, seeds ? seeds + base : nullptr, out + base,
+                             palettes ? palettes + (size_t)base * NQ_MAXK : nullptr, plens ? plens + base : nullptr,
+                             hasAlpha ? hasAlpha + base : nullptr);
+  });
 }
 
 int nq_convert(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax, int dither, uint64_t seed, uint32_t* out,
@@ -1123,30 +1263,20 @@ int nq_dither_with_palette(nq_ctx* c, int kind, const uint32_t* in, int w, int h
   if (rc) return rc;
   if (!palette || plen <= 0 || plen > NQ_MAXK) return fail(NQ_ERR_ARG, "palette_len must be 1..256");
   CU(cudaSetDevice(c->device));
-  const size_t bytes = (size_t)w * h * 4;
-  rc = ensure_stage(c, bytes);
-  if (rc) return rc;
   DevBuf dPal;
   CU(dPal.alloc(NQ_MAXK * 4));
   CU(cudaMemcpy(dPal.p, palette, (size_t)plen * 4, cudaMemcpyHostToDevice));
-  rc = convert_device(c, kind, c->dIn, 1, w, h, nmax, dither, &seed, c->dOut, nullptr, nullptr, nullptr, dPal.as<uint32_t>(), plen, in, out);
-  if (rc) return rc;
-  CU(cudaStreamSynchronize(c->stream));
-  return NQ_OK;
+  return convert_host(c, kind, 1, &w, &h, &in, &out, nmax, dither, &seed, nullptr, nullptr, nullptr, dPal.as<uint32_t>(), plen);
 }
 
 int nq_histogram(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax, int* nBins, double* bins5, float* initErr, int* initNn, int capacity) {
   int rc = check_args(c, kind, in, 1, w, h, nmax, in);
   if (rc) return rc;
   if (!nBins) return fail(NQ_ERR_ARG, "n_bins must not be null");
-  CU(cudaSetDevice(c->device));
-  const size_t bytes = (size_t)w * h * 4;
-  rc = ensure_stage(c, bytes);
-  if (rc) return rc;
   const bool wasDebug = c->debug;
   c->debug = true;                                   // the hook returns what debug mode records after the find_nn sweep
   uint64_t seed = 0;
-  rc = convert_device(c, kind, c->dIn, 1, w, h, nmax, 1, &seed, c->dOut, nullptr, nullptr, nullptr, nullptr, 0, in, nullptr, true);
+  rc = convert_host(c, kind, 1, &w, &h, &in, nullptr, nmax, 1, &seed, nullptr, nullptr, nullptr, nullptr, 0, true);
   c->debug = wasDebug;
   if (rc) return rc;
   const DebugImage& D = c->dbg[0];
@@ -1161,9 +1291,13 @@ int nq_histogram(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax
 
 int nq_gilbert_order(int w, int h, uint32_t* out) {
   if (w <= 0 || h <= 0 || !out) return fail(NQ_ERR_ARG, "bad arguments");
-  size_t n = 0;
-  gilbert_walk(w, h, [&](int x, int y) { out[n++] = (uint32_t)(x + y * w); });
-  return n == (size_t)w * h ? NQ_OK : fail(NQ_ERR_ARG, "gilbert walk size mismatch");
+  const unsigned long long npix = (unsigned long long)w * (unsigned long long)h;
+  for (unsigned long long n = 0; n < npix; ++n) {
+    int x, y;
+    nq::gilbert_xy(w, h, n, &x, &y);
+    out[n] = (uint32_t)(x + y * w);
+  }
+  return NQ_OK;
 }
 
 int nq_get_image_info(nq_ctx* c, int image, nq_image_info* o) {

@@ -973,13 +973,14 @@ __device__ uint32_t prelookup_commit(Env& E, uint32_t c, bool mine) {
 }
 
 // `want`: which images this launch takes by NqImage::specDone: 0 = not the speculative path's, 3 = handed back by it
-__global__ void __launch_bounds__(64) k_dither_fifo(NqImage* imgs, const NqSlot* slots, const uint32_t* order, int cacheBytes, int want) {
+__global__ void __launch_bounds__(64) k_dither_fifo(NqImage* imgs, const NqSlot* slots, int cacheBytes, int want) {
   __shared__ WarpShared sh;
   __shared__ DitherRing ring;
   extern __shared__ unsigned short dynCache[];     // 16 384 entries when launched with cacheBytes, else nothing
   const int img = blockIdx.x;
   NqImage& I = imgs[img];
   const NqSlot& S = slots[img];
+  const uint32_t* order = S.order;
   const unsigned lane = lane_id();
   const int plen = I.paletteLen;
   if (plen <= 0 || I.error || I.gSorted || I.specDone != want) return;
@@ -1235,12 +1236,13 @@ struct PQ {
   }
 };
 
-__global__ void __launch_bounds__(32) k_dither_sorted(NqImage* imgs, const NqSlot* slots, const uint32_t* order) {
+__global__ void __launch_bounds__(32) k_dither_sorted(NqImage* imgs, const NqSlot* slots) {
   __shared__ WarpShared sh;
   __shared__ SortedShared qs;
   const int img = blockIdx.x;
   NqImage& I = imgs[img];
   const NqSlot& S = slots[img];
+  const uint32_t* order = S.order;
   const unsigned lane = lane_id();
   const int plen = I.paletteLen;
   if (plen <= 0 || I.error || !I.gSorted) return;

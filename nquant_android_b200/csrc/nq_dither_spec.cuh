@@ -1085,7 +1085,9 @@ struct SpecImage {
 #define NQS_ACTIVE(P) ((P).eligible && !(P).W.state[1])
 #define NQS_CHUNK 8192           // pixels per block of the draw-count prefix sum (stage 2)
 
-// GilbertCurve / quantizer constants of every image, and which images this path takes (one thread per image)
+// GilbertCurve / quantizer constants of every image, and which images this path takes (one thread per image).
+// order: nullptr = every image walks its slot's own table (NqSlot::order); else one table for every image of the list (the
+// CPU emulation of these kernels, tests/spec_host_harness.cpp, runs one size).
 __global__ void k_spec_setup(NqImage* imgs, const NqSlot* slots, SpecImage* sp, const uint32_t* order, int nimg, int seg, int warm, int* eligOut) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= nimg) return;
@@ -1120,7 +1122,7 @@ __global__ void k_spec_setup(NqImage* imgs, const NqSlot* slots, SpecImage* sp, 
   C.opaque = opaque;
   // which instantiation of stage 6 runs this image: bits 8.. of the verdict (spec_drive groups the images by it)
   eligOut[i] |= (((C.DM == 25 ? 2 : (C.DM == 16 ? 1 : 0)) << 1) | (opaque ? 0 : 1)) << 8;
-  P.W.order = order; P.W.in = slots[i].in; P.W.out = slots[i].out; P.W.cells = slots[i].cells;
+  P.W.order = order ? order : slots[i].order; P.W.in = slots[i].in; P.W.out = slots[i].out; P.W.cells = slots[i].cells;
   P.W.lut = g_gammaLut; P.W.bn = g_blueNoise;
   fill_tables(C, g_gammaLut);
 }

@@ -74,6 +74,7 @@ struct NqSlot {
   uint2* heap;                     // [65538] global spill of the lower heap levels: {err bits, id | nn << 16}
   int* mergeLog;                   // optional [2*65536] (tb, nb) pairs for parity tests
   // dither
+  const uint32_t* order;           // [npix] Gilbert visiting order of the image's size, x | y << 16 (shared by equal sizes)
   unsigned short* memo;            // [65536] nearestMap for reduced keys (0xFFFF = absent)
   unsigned short* idx;             // [npix] palette indices of pass 1 when a second pass follows
   unsigned char* cells;            // [32768][32] candidate lists of the CIELAB closest-colour scan (k_build_cells)

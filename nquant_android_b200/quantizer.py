@@ -80,6 +80,26 @@ class Context:
         self._check(fn(self._h, kind, ctypes.c_void_p(in_ptr), n, width, height, int(n_max_colors), int(bool(dither)),
                        _p(sd), ctypes.c_void_p(out_ptr), _p(palettes), _p(palette_lens), None))
 
+    def convert_ragged(self, kind, images, n_max_colors, dither, seeds=None):
+        """nq_convert_ragged: images of different sizes in one call. images: list of (height, width) uint32 host arrays.
+        Returns (list of (height, width) outputs, palettes (n, 256), palette_lens, has_alpha)."""
+        R = _Ragged(images)
+        sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._check(self._L.nq_convert_ragged(self._h, kind, R.in_ptrs, _p(R.widths), _p(R.heights), R.n, int(n_max_colors),
+                                              int(bool(dither)), _p(sd), R.out_ptrs, _p(R.pal), _p(R.plen), _p(R.ha)))
+        return R.outs, R.pal, R.plen, R.ha
+
+    def convert_ragged_ptr(self, kind, in_ptr, out_ptr, widths, heights, n_max_colors, dither, seeds=None, palettes=None,
+                           palette_lens=None, has_alpha=None):
+        """nq_convert_ragged_device: device buffers (e.g. torch tensors) holding the images packed back to back, image i
+        widths[i] x heights[i] pixels. palettes / palette_lens / has_alpha: optional host arrays that receive the results."""
+        w = np.ascontiguousarray(widths, dtype=np.int32)
+        h = np.ascontiguousarray(heights, dtype=np.int32)
+        sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._check(self._L.nq_convert_ragged_device(self._h, kind, ctypes.c_void_p(in_ptr), _p(w), _p(h), len(w), int(n_max_colors),
+                                                     int(bool(dither)), _p(sd), ctypes.c_void_p(out_ptr), _p(palettes), _p(palette_lens),
+                                                     _p(has_alpha)))
+
     def dither_with_palette(self, kind, argb, width, height, n_max_colors, dither, palette, seed=0):
         argb = np.ascontiguousarray(argb, dtype=np.uint32)
         palette = np.ascontiguousarray(palette, dtype=np.uint32)
@@ -211,6 +231,38 @@ def convert_batch_multi(contexts, kind, argb, width, height, n_max_colors, dithe
     if rc != 0:
         raise NQuantError(rc, L.nq_last_error().decode())
     return out, pal, plen, ha
+
+
+class _Ragged:
+    """Host arguments of the ragged entry points: sides, per-image pointer arrays, result arrays."""
+
+    def __init__(self, images):
+        self.ins = [np.ascontiguousarray(im, dtype=np.uint32) for im in images]
+        if any(im.ndim != 2 for im in self.ins):
+            raise NQuantError(_lib.NQ_ERR_ARG, "every image must be a (height, width) array")
+        self.n = len(self.ins)
+        self.heights = np.array([im.shape[0] for im in self.ins], dtype=np.int32)
+        self.widths = np.array([im.shape[1] for im in self.ins], dtype=np.int32)
+        self.outs = [np.empty_like(im) for im in self.ins]
+        self.in_ptrs = (ctypes.c_void_p * self.n)(*[im.ctypes.data for im in self.ins])
+        self.out_ptrs = (ctypes.c_void_p * self.n)(*[o.ctypes.data for o in self.outs])
+        self.pal = np.zeros((self.n, 256), dtype=np.uint32)
+        self.plen = np.zeros(self.n, dtype=np.int32)
+        self.ha = np.zeros(self.n, dtype=np.int32)
+
+
+def convert_ragged_multi(contexts, kind, images, n_max_colors, dither, seeds=None, queue_images=0):
+    """nq_convert_ragged_multi: images of different sizes over several contexts, pieces of `queue_images` images handed out
+    dynamically (0 = one piece per context). Returns (list of outputs, palettes, palette_lens, has_alpha)."""
+    L = _lib.load()
+    R = _Ragged(images)
+    sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+    handles = (ctypes.c_void_p * len(contexts))(*[c._h for c in contexts])
+    rc = L.nq_convert_ragged_multi(handles, len(contexts), kind, R.in_ptrs, _p(R.widths), _p(R.heights), R.n, int(n_max_colors),
+                                   int(bool(dither)), _p(sd), R.out_ptrs, _p(R.pal), _p(R.plen), _p(R.ha), int(queue_images))
+    if rc != 0:
+        raise NQuantError(rc, L.nq_last_error().decode())
+    return R.outs, R.pal, R.plen, R.ha
 
 
 def default_context(device=0):
