@@ -124,6 +124,29 @@ int nq_convert_ragged_device(nq_ctx* ctx, int kind, const uint32_t* d_argb_in, c
                              int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds, uint32_t* d_argb_out,
                              uint32_t* palettes_out, int* palette_lens, int* has_alpha);
 
+/* nq_convert_ragged with an INDEX MAP: the palette index of every output pixel, one byte per pixel, computed on the GPU
+ * from the finished output -- what an indexed format (PNG8, GIF, a palette texture) stores, at a quarter of the bytes of
+ * the colours. index_out[i] receives widths[i]*heights[i] bytes, row-major like the pixels. argb_out may be NULL: the
+ * colours are then not copied back at all; otherwise argb_out[i] receives them as in nq_convert_ragged.
+ * The index of a pixel is the LOWEST palette index whose colour equals the output pixel, so
+ * palettes_out[i*256 + index] == argb_out[i][p] always holds; with distinct palette colours (every palette the two
+ * quantizers are known to produce) it is the index the reference's own lookup chose (GilbertCurve.java:278-279). Colours
+ * are whole 0xAARRGGBB words: entries that differ in alpha only are different colours. n_max_colors <= 256, so an index
+ * fits in a byte. Everything else -- palettes, palette_lens, has_alpha, nq_get_image_info, errors, streams and chunking --
+ * is as in nq_convert_ragged; an equal-size batch is the case widths[i] == width, heights[i] == height. A NULL index_out or
+ * a NULL entry in it returns NQ_ERR_ARG before any work. */
+int nq_convert_ragged_indexed(nq_ctx* ctx, int kind, const uint32_t* const* argb_in, const int* widths, const int* heights,
+                              int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds,
+                              uint8_t* const* index_out, uint32_t* const* argb_out, uint32_t* palettes_out, int* palette_lens,
+                              int* has_alpha);
+
+/* The same with DEVICE buffers on the context's GPU, as in nq_convert_ragged_device. d_index_out is packed too: image i's
+ * indices start at byte sum_{j<i} widths[j]*heights[j]. d_argb_out may be NULL: the colours then go to scratch memory of
+ * the context (kept for its next calls). Every device base pointer must be 16-byte aligned (NQ_ERR_ARG otherwise). */
+int nq_convert_ragged_indexed_device(nq_ctx* ctx, int kind, const uint32_t* d_argb_in, const int* widths, const int* heights,
+                                     int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds, uint8_t* d_index_out,
+                                     uint32_t* d_argb_out, uint32_t* palettes_out, int* palette_lens, int* has_alpha);
+
 /* nq_convert_ragged over several contexts with the dynamic queue of nq_convert_batch_multi (pieces of queue_images
  * images, 0 = one piece per context). */
 int nq_convert_ragged_multi(nq_ctx** contexts, int n_contexts, int kind, const uint32_t* const* argb_in, const int* widths,

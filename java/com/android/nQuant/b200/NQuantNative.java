@@ -48,6 +48,10 @@ final class NQuantNative {
 	//                             rng_seeds, argb_out[], palettes_out, palette_lens, has_alpha, queue_images): images of different sizes
 	static final MethodHandle nq_convert_ragged_multi = h("nq_convert_ragged_multi",
 		FunctionDescriptor.of(I, P, I, I, P, P, P, I, I, I, P, P, P, P, P, I));
+	// int nq_convert_ragged_indexed(ctx, kind, argb_in[], widths, heights, n_images, n_max_colors, dither, rng_seeds,
+	//                               index_out[], argb_out[] (NULL: colours not returned), palettes_out, palette_lens, has_alpha)
+	static final MethodHandle nq_convert_ragged_indexed = h("nq_convert_ragged_indexed",
+		FunctionDescriptor.of(I, P, I, P, P, P, I, I, I, P, P, P, P, P, P));
 	// int nq_device_count(void)
 	static final MethodHandle nq_device_count = h("nq_device_count", FunctionDescriptor.of(I));
 	// int nq_set_spec_dither(ctx, on, segment, warmup): speculative segment-parallel error diffusion, on by default (DESIGN.md 7.1)

@@ -71,6 +71,41 @@ public class PnnQuantizer implements AutoCloseable {
 		}
 	}
 
+	/**
+	 * convert() as palette indices, one byte per pixel, computed on the GPU (nq_convert_ragged_indexed): what an indexed
+	 * format (PNG8, GIF, a palette texture) stores. getPalette()[index & 0xFF] is the colour convert() returns for the pixel
+	 * (the lowest index of that colour). The colours themselves are not copied back. Sets getPalette() and hasAlpha() like
+	 * convert().
+	 */
+	public byte[] convertIndexed(int nMaxColors, boolean dither) throws Exception {
+		try (Arena arena = Arena.ofConfined()) {
+			final long n = (long) width * height;
+			MemorySegment in = arena.allocate(ValueLayout.ADDRESS);
+			in.set(ValueLayout.ADDRESS, 0, arena.allocateFrom(ValueLayout.JAVA_INT, pixels));
+			MemorySegment idx = arena.allocate(n);
+			MemorySegment idxs = arena.allocate(ValueLayout.ADDRESS);
+			idxs.set(ValueLayout.ADDRESS, 0, idx);
+			MemorySegment w = arena.allocateFrom(ValueLayout.JAVA_INT, width);
+			MemorySegment h = arena.allocateFrom(ValueLayout.JAVA_INT, height);
+			MemorySegment seed = arena.allocateFrom(ValueLayout.JAVA_LONG, rngSeed);
+			MemorySegment pal = arena.allocate(ValueLayout.JAVA_INT, 256);
+			MemorySegment plen = arena.allocate(ValueLayout.JAVA_INT);
+			MemorySegment alpha = arena.allocate(ValueLayout.JAVA_INT);
+			int rc;
+			try {
+				rc = (int) NQuantNative.nq_convert_ragged_indexed.invokeExact(NQuantNative.context(device), kind(), in, w, h, 1, nMaxColors,
+					dither ? 1 : 0, seed, idxs, MemorySegment.NULL, pal, plen, alpha);
+			} catch (Throwable t) {
+				throw new Exception(t);
+			}
+			if (rc != 0)
+				throw new Exception("nq_convert_ragged_indexed failed (" + rc + "): " + NQuantNative.lastError());
+			hasAlpha = alpha.get(ValueLayout.JAVA_INT, 0) != 0;
+			palette = pal.asSlice(0, 4L * plen.get(ValueLayout.JAVA_INT, 0)).toArray(ValueLayout.JAVA_INT);
+			return idx.toArray(ValueLayout.JAVA_BYTE);
+		}
+	}
+
 	/** boolean hasAlpha() (PnnQuantizer.java:458). */
 	public boolean hasAlpha() {
 		return hasAlpha;

@@ -7,7 +7,7 @@ CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libnquant_b200.so")
 SOURCES = ["nq_api.cu"]
 DEPS = ["nq_api.cu", "nq_types.h", "nq_math.h", "nq_math_tables.h", "nq_color.h", "nq_bluenoise_table.h",
-        "nq_hist.cuh", "nq_pnn.cuh", "nq_dither.cuh", "nq_dither_spec.cuh", "nq_fastmath.cuh", "nq_gilbert.h", os.path.join("..", "..", "include", "nquant_b200.h")]
+        "nq_hist.cuh", "nq_pnn.cuh", "nq_dither.cuh", "nq_dither_spec.cuh", "nq_fastmath.cuh", "nq_gilbert.h", "nq_index.h", os.path.join("..", "..", "include", "nquant_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

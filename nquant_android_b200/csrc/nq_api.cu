@@ -25,6 +25,7 @@
 #include "nq_dither.cuh"
 #include "nq_dither_spec.cuh"
 #include "nq_gilbert.h"
+#include "nq_index.h"
 
 #define NQ_NSTAGES 6   // scan, histogram, find_nn sweep, merge, dither setup + saliency, dither
 #define NQ_NKERNELS 4  // kernels timed on their own (nq_get_kernel_times): 0 k_spec_run, 1 k_dither_fifo, 2 k_dither_sorted, 3 k_merge_*
@@ -59,6 +60,47 @@ __global__ void k_gilbert_order(const GilbertJob* jobs, int njobs) {
       J.dst[n] = (uint32_t)x | ((uint32_t)y << 16);
     }
   }
+}
+
+// ---- index map of the finished output (nq_convert_ragged_indexed*), one byte per pixel: the rule is in nq_index.h --------
+#define NQ_DEVERR_INDEX 5   // NqImage::error: an output pixel whose colour is not in the image's palette
+// One pass over the image's ARGB output; blockIdx.y = image. A thread reads 4 pixels as one 16-byte vector and writes their
+// 4 index bytes as one word, at the pixel positions of the call that are multiples of 4: the call's ARGB and index planes
+// are 16-byte aligned at their bases and hold image i at the same pixel offset, so both accesses are aligned there. The
+// pixels before the image's first such position and after its last go one by one. A colour missing from the palette cannot
+// happen by construction; if one does, the image's error is set and the call fails. Images already in error are skipped.
+__global__ void __launch_bounds__(256) k_index_map(NqImage* imgs, const NqSlot* slots) {
+  __shared__ unsigned long long tab[NQ_IMAP_SLOTS];
+  __shared__ uint32_t pal[NQ_MAXK];
+  NqImage& I = imgs[blockIdx.y];
+  if (I.error) return;
+  const int plen = I.paletteLen, npix = I.npix;
+  for (int k = threadIdx.x; k < NQ_IMAP_SLOTS; k += blockDim.x) tab[k] = NQ_IMAP_EMPTY;
+  for (int k = threadIdx.x; k < plen; k += blockDim.x) pal[k] = I.palette[k];
+  __syncthreads();
+  for (int k = threadIdx.x; k < plen; k += blockDim.x) nq::imap_insert(tab, pal, k);
+  __syncthreads();
+  const uint32_t* out = slots[blockIdx.y].out;
+  unsigned char* idx = slots[blockIdx.y].index;
+  const int head = min(npix, (int)((16 - ((uintptr_t)out & 15)) & 15) / 4);
+  const int nvec = (npix - head) / 4, tail = head + 4 * nvec;
+  const int t0 = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
+  int miss = 0;
+  const uint4* src = reinterpret_cast<const uint4*>(out + head);
+  uint32_t* dst = reinterpret_cast<uint32_t*>(idx + head);
+  for (int v = t0; v < nvec; v += nt) {
+    const uint4 q = __ldcs(src + v);   // streaming: every pixel is read once (and ld.global: the pointer comes from a struct)
+    const int a = nq::imap_lookup(tab, q.x), b = nq::imap_lookup(tab, q.y), c = nq::imap_lookup(tab, q.z), d = nq::imap_lookup(tab, q.w);
+    miss |= a | b | c | d;
+    __stcs(dst + v, (uint32_t)(a & 255) | (uint32_t)(b & 255) << 8 | (uint32_t)(c & 255) << 16 | (uint32_t)(d & 255) << 24);
+  }
+  for (int r = t0; r < head + (npix - tail); r += nt) {
+    const int p = r < head ? r : tail + (r - head);
+    const int a = nq::imap_lookup(tab, out[p]);
+    miss |= a;
+    idx[p] = (unsigned char)a;
+  }
+  if (miss < 0) atomicCAS(&I.error, 0, NQ_DEVERR_INDEX);
 }
 
 // ---- synthetic images (nquant_android_b200/synth.py) ---------------------------------------------
@@ -188,10 +230,10 @@ struct nq_ctx {
   int wsSlots = 0, wsNpix = 0, wsKind = -1, sortSets = 0;
   bool wsDebug = false, wsBits = false, wsIdx = false;
   std::vector<NqSlot> hSlots;
-  // staging for host-buffer calls
+  // staging for host-buffer calls; dOut alone is the ARGB scratch of device index-map calls that want no colours back
   uint32_t* dIn = nullptr;
   uint32_t* dOut = nullptr;
-  size_t stageBytes = 0;
+  size_t inBytes = 0, outBytes = 0;
   // per-stage device timing (CUDA events on the internal streams, summed over the chunks of a call)
   double stageMs[NQ_NSTAGES] = {};
   unsigned long long stageLaunches[NQ_NSTAGES] = {};
@@ -414,8 +456,12 @@ struct GroupArgs {
   const uint32_t* dPalIn;
   int palInLen;
   const uint32_t* const* hIn;       // host pixels of each image (nullptr: dIn is the caller's device buffer and already holds them)
-  uint32_t* const* hOut;
+  uint32_t* const* hOut;            // (nullptr: no host copy of the colours)
   bool stopAfterSweep = false;      // stage hook nq_histogram: no merge loop, no dither
+  // index-map calls: the call's packed index plane, image i at byte off[i] (nullptr: no index map), and the host
+  // destination of each image's indices (nullptr: the plane is the caller's device buffer)
+  unsigned char* dIdx = nullptr;
+  uint8_t* const* hIdx = nullptr;
 };
 
 int max_npix(const GroupArgs& A, int base, int n) {
@@ -442,6 +488,21 @@ cudaError_t copy_out(const GroupArgs& A, int from, int to, const uint32_t* dOut,
   }
   return cudaSuccess;
 }
+cudaError_t copy_indices(const GroupArgs& A, int from, int to, cudaStream_t st) {
+  for (int i = from, j; i < to; i = j) {
+    for (j = i + 1; j < to && A.hIdx[j] == A.hIdx[i] + (A.off[j] - A.off[i]); ++j) {}
+    cudaError_t e = cudaMemcpyAsync(A.hIdx[i], A.dIdx + A.off[i], A.off[j] - A.off[i], cudaMemcpyDeviceToHost, st);
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
+
+// k_index_map over images [from, to) of the group, whose dither is complete in the order of stream `st`
+cudaError_t enqueue_index_map(nq_ctx* c, const GroupArgs& A, int from, int to, cudaStream_t st) {
+  const int n = to - from;
+  k_index_map<<<dim3(pixel_grid_x(c, max_npix(A, from, n), n), n), 256, 0, st>>>(c->dImgs + from, c->dSlots + from); ++c->launches;
+  return cudaGetLastError();
+}
 
 // One chunk of a call: images [base, base + n) of the group, with the events that bracket its stages.
 struct Chunk {
@@ -457,7 +518,7 @@ struct Chunk {
   unsigned long long launches[NQ_NSTAGES] = {};
   // host-buffer calls: images [0, copied) of the chunk are already on their way to the host (progressive copy-out)
   int copied = 0;
-  const GroupArgs* A = nullptr;    // the group's host destinations (GroupArgs::hOut), or nullptr
+  const GroupArgs* A = nullptr;    // the group, when it has host destinations (GroupArgs::hOut, hIdx); else nullptr
   const uint32_t* dOut = nullptr;  // the call's packed device output
 };
 
@@ -503,12 +564,16 @@ struct SpecCudaBackend {
     cudaEventRecord(t0, st);
   }
   // images [0, prefix) of the chunk are complete: copy them out on the copy-out stream while the rest is still being dithered
+  // (an index-map call computes their indices first, here on the dither stream)
   void done_prefix(int prefix) {
     if (!ch->A || prefix - ch->copied < 16) return;
+    const GroupArgs& A = *ch->A;
+    if (A.dIdx) keep(enqueue_index_map(c, A, ch->base + ch->copied, ch->base + prefix, st));
     cudaEvent_t e = take_event(c);
     keep(cudaEventRecord(e, st));
     keep(cudaStreamWaitEvent(c->sOut, e, 0));
-    keep(copy_out(*ch->A, ch->base + ch->copied, ch->base + prefix, ch->dOut, c->sOut));
+    if (A.hOut) keep(copy_out(A, ch->base + ch->copied, ch->base + prefix, ch->dOut, c->sOut));
+    if (A.hIdx) keep(copy_indices(A, ch->base + ch->copied, ch->base + prefix, c->sOut));
     ch->copied = prefix;
   }
   void note(int round, int active, int open, int patches, int redos) {
@@ -624,6 +689,7 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
     S.in = dIn + A.off[g];
     S.out = dOut + A.off[g];
     S.order = A.order ? A.order[g] : nullptr;
+    S.index = A.dIdx ? A.dIdx + A.off[g] : nullptr;
     if (kind == NQ_KIND_LAB) {   // sort scratch: the sets of this chunk's front stream, cycled through the chunk
       unsigned char* sp = c->sortPool + c->sortSetBytes * ((size_t)ch.frontIdx * c->sortSets + (size_t)(i % c->sortSets));
       S.sortA = reinterpret_cast<uint32_t*>(sp);
@@ -891,13 +957,20 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
       for (auto& e : chunks[k].evD) CU(cudaEventRecord(e, c->sDith));
       continue;
     }
-    if (A.hOut) { chunks[k].A = &G; chunks[k].dOut = dOut; }
+    if (A.hOut || A.hIdx) { chunks[k].A = &G; chunks[k].dOut = dOut; }
     rc = run_dither(c, chunks[k], G);
     if (rc) return rc;
-    if (A.hOut && chunks[k].copied < chunks[k].n) {   // device -> host of what the progressive copy-out has not taken yet
-      Chunk& ch = chunks[k];
-      CU(cudaStreamWaitEvent(c->sOut, ch.evD[2], 0));
-      CU(copy_out(A, ch.base + ch.copied, ch.base + ch.n, dOut, c->sOut));
+    Chunk& ch = chunks[k];
+    cudaEvent_t evDone = ch.evD[2];
+    if (A.dIdx && ch.copied < ch.n) {   // indices of what the progressive copy-out has not taken yet
+      CU(enqueue_index_map(c, A, ch.base + ch.copied, ch.base + ch.n, c->sDith));
+      evDone = take_event(c);
+      CU(cudaEventRecord(evDone, c->sDith));
+    }
+    if ((A.hOut || A.hIdx) && ch.copied < ch.n) {   // device -> host of what the progressive copy-out has not taken yet
+      CU(cudaStreamWaitEvent(c->sOut, evDone, 0));
+      if (A.hOut) CU(copy_out(A, ch.base + ch.copied, ch.base + ch.n, dOut, c->sOut));
+      if (A.hIdx) CU(copy_indices(A, ch.base + ch.copied, ch.base + ch.n, c->sOut));
     }
   }
   CU(cudaEventRecord(evOut, c->sOut));
@@ -940,10 +1013,12 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
 
 // Every convert entry point, equal sizes or not, ends here. Image i is ws[i] x hs[i] pixels; dIn / dOut: device buffers of
 // the whole call, the images packed back to back. hIn / hOut (optional): one host pointer per image, read from / written to
-// chunk by chunk, overlapped with the kernels. The workspace is sized by the largest image of the call.
+// chunk by chunk, overlapped with the kernels. The workspace is sized by the largest image of the call. dIdx (optional): the
+// index plane, image i at byte off[i], filled by k_index_map; hIdx (optional): one host pointer per image it is copied to.
 int convert_device(nq_ctx* c, int kind, int n, const int* ws, const int* hs, const uint32_t* dIn, uint32_t* dOut, int nmax, int dither,
                    const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn, int palInLen,
-                   const uint32_t* const* hIn = nullptr, uint32_t* const* hOut = nullptr, bool stopAfterSweep = false) {
+                   const uint32_t* const* hIn = nullptr, uint32_t* const* hOut = nullptr, bool stopAfterSweep = false,
+                   unsigned char* dIdx = nullptr, uint8_t* const* hIdx = nullptr) {
   CU(cudaSetDevice(c->device));
   std::vector<size_t> off(n + 1, 0);
   int npix = 1;
@@ -965,6 +1040,8 @@ int convert_device(nq_ctx* c, int kind, int n, const int* ws, const int* hs, con
     GroupArgs A{kind, nmax, dither, ws + base, hs + base, off.data() + base, order.empty() ? nullptr : order.data() + base,
                 seeds ? seeds + base : nullptr, dPalIn, palInLen, hIn ? hIn + base : nullptr, hOut ? hOut + base : nullptr};
     A.stopAfterSweep = stopAfterSweep;
+    A.dIdx = dIdx;
+    A.hIdx = hIdx ? hIdx + base : nullptr;
     rc = convert_group(c, A, m, dIn, dOut, base);
     if (rc) return rc;
     collect_results(c, base, m, palettes, plens, hasAlpha, &firstErr);
@@ -973,33 +1050,41 @@ int convert_device(nq_ctx* c, int kind, int n, const int* ws, const int* hs, con
   c->lastImgs.swap(all);
   if (firstErr == 3) return fail(NQ_ERR_COLOR, "alpha must be between 0 and 255. (ColorUtils.setAlphaComponent)");
   if (firstErr == 4) return fail(NQ_ERR_UNSUPPORTED, "PnnLABQuantizer with dither == false, more than 32 colours and semi-transparent pixels is not covered");
+  if (firstErr == NQ_DEVERR_INDEX) return fail(NQ_ERR_CUDA, "index map: an output pixel's colour is not in its image's palette (internal error)");
   if (firstErr) return fail(NQ_ERR_UNSUPPORTED, "device-side error " + std::to_string(firstErr));
   return NQ_OK;
 }
 
-int ensure_stage(nq_ctx* c, size_t bytes) {
-  if (c->stageBytes >= bytes) return NQ_OK;
+int ensure_buffer(uint32_t** buf, size_t* have, size_t bytes) {
+  if (*have >= bytes) return NQ_OK;
   CU(cudaDeviceSynchronize());
-  if (c->dIn) cudaFree(c->dIn);
-  if (c->dOut) cudaFree(c->dOut);
-  c->dIn = c->dOut = nullptr; c->stageBytes = 0;
-  CU(cudaMalloc(&c->dIn, bytes));
-  cudaError_t e = cudaMalloc(&c->dOut, bytes);
-  if (e != cudaSuccess) { cudaFree(c->dIn); c->dIn = nullptr; return fail(NQ_ERR_NOMEM, std::string("cudaMalloc(staging): ") + cudaGetErrorString(e)); }
-  c->stageBytes = bytes;
+  if (*buf) cudaFree(*buf);
+  *buf = nullptr; *have = 0;
+  cudaError_t e = cudaMalloc(buf, bytes);
+  if (e != cudaSuccess) { *buf = nullptr; return fail(NQ_ERR_NOMEM, std::string("cudaMalloc(staging): ") + cudaGetErrorString(e)); }
+  *have = bytes;
   return NQ_OK;
 }
+int ensure_stage(nq_ctx* c, size_t bytes) {
+  int rc = ensure_buffer(&c->dIn, &c->inBytes, bytes);
+  return rc ? rc : ensure_buffer(&c->dOut, &c->outBytes, bytes);
+}
 
-// host-buffer calls: the images go through the context's staging buffers (sized by the call's total pixels)
+// host-buffer calls: the images go through the context's staging buffers (sized by the call's total pixels). The index plane
+// of an index-map call (idx: one host pointer per image) overlays the input staging: image i's indices take bytes
+// [off[i], off[i+1]), which lie inside the input of images 0..i, and k_index_map writes them only once images 0..i are
+// complete (after the chunk's dither, or for the complete prefix the progressive copy-out hands on), so no kernel reads
+// that input again. Later images' input starts at byte 4 * off[i+1] or later and stays intact.
 int convert_host(nq_ctx* c, int kind, int n, const int* ws, const int* hs, const uint32_t* const* in, uint32_t* const* out, int nmax,
                  int dither, const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn = nullptr,
-                 int palInLen = 0, bool stopAfterSweep = false) {
+                 int palInLen = 0, bool stopAfterSweep = false, uint8_t* const* idx = nullptr) {
   CU(cudaSetDevice(c->device));
   size_t total = 0;
   for (int i = 0; i < n; ++i) total += (size_t)ws[i] * hs[i];
   int rc = ensure_stage(c, total * 4);
   if (rc) return rc;
-  rc = convert_device(c, kind, n, ws, hs, c->dIn, c->dOut, nmax, dither, seeds, palettes, plens, hasAlpha, dPalIn, palInLen, in, out, stopAfterSweep);
+  rc = convert_device(c, kind, n, ws, hs, c->dIn, c->dOut, nmax, dither, seeds, palettes, plens, hasAlpha, dPalIn, palInLen, in, out, stopAfterSweep,
+                      idx ? reinterpret_cast<unsigned char*>(c->dIn) : nullptr, idx);
   if (rc) return rc;
   CU(cudaStreamSynchronize(c->stream));
   return NQ_OK;
@@ -1224,6 +1309,32 @@ int nq_convert_ragged(nq_ctx* c, int kind, const uint32_t* const* in, const int*
   if (rc) return rc;
   NvtxRange nv("nq_convert_ragged");
   return convert_host(c, kind, n, ws, hs, in, out, nmax, dither, seeds, palettes, plens, hasAlpha);
+}
+
+int nq_convert_ragged_indexed(nq_ctx* c, int kind, const uint32_t* const* in, const int* ws, const int* hs, int n, int nmax, int dither,
+                              const uint64_t* seeds, uint8_t* const* idx, uint32_t* const* out, uint32_t* palettes, int* plens, int* hasAlpha) {
+  int rc = check_ragged(c, kind, in, ws, hs, n, nmax, idx, in, out);
+  if (rc) return rc;
+  for (int i = 0; i < n; ++i)
+    if (!idx[i]) return fail(NQ_ERR_ARG, "image " + std::to_string(i) + ": null index buffer");
+  NvtxRange nv("nq_convert_ragged_indexed");
+  return convert_host(c, kind, n, ws, hs, in, out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0, false, idx);
+}
+
+int nq_convert_ragged_indexed_device(nq_ctx* c, int kind, const uint32_t* d_in, const int* ws, const int* hs, int n, int nmax, int dither,
+                                     const uint64_t* seeds, uint8_t* d_idx, uint32_t* d_out, uint32_t* palettes, int* plens, int* hasAlpha) {
+  int rc = check_ragged(c, kind, d_in, ws, hs, n, nmax, d_idx);
+  if (rc) return rc;
+  if (((uintptr_t)d_in | (uintptr_t)d_idx | (uintptr_t)d_out) & 15) return fail(NQ_ERR_ARG, "device buffers must be 16-byte aligned");
+  NvtxRange nv("nq_convert_ragged_indexed_device");
+  if (!d_out) {   // the colours stay in the context's scratch
+    CU(cudaSetDevice(c->device));
+    size_t total = 0;
+    for (int i = 0; i < n; ++i) total += (size_t)ws[i] * hs[i];
+    if ((rc = ensure_buffer(&c->dOut, &c->outBytes, total * 4))) return rc;
+    d_out = c->dOut;
+  }
+  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0, nullptr, nullptr, false, d_idx);
 }
 
 int nq_convert_batch_multi(nq_ctx** ctxs, int nctx, int kind, const uint32_t* in, int n, int w, int h, int nmax, int dither,

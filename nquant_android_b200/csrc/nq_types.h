@@ -80,4 +80,5 @@ struct NqSlot {
   unsigned char* cells;            // [32768][32] candidate lists of the CIELAB closest-colour scan (k_build_cells)
   unsigned int* bits;              // [2^27] one bit per ARGB colour ever passed to getLab (pixelMap, PL:34-42); only when the
                                    // BlueNoise second pass needs pixelMap.size() (PL:511-513)
+  unsigned char* index;            // [npix] palette index of every output pixel (k_index_map); only in the index-map calls
 };

@@ -44,8 +44,18 @@ def _chunk(tag, data):
 
 def write_indexed_png(path, out_argb, palette, width, height, level=6):
     """Write the quantized image as an 8-bit indexed PNG (colour type 3). Alpha goes to a tRNS chunk."""
-    idx = to_indices(out_argb, palette).reshape(height, width)
+    return write_png8(path, to_indices(out_argb, palette), palette, width, height, level)
+
+
+def write_png8(path, indices, palette, width, height, level=6):
+    """Write an index map (one uint8 palette index per pixel, row-major, e.g. from Context.convert_indexed) and its palette
+    as an 8-bit indexed PNG (colour type 3). Alpha goes to a tRNS chunk. Returns the file's size in bytes."""
+    idx = np.ascontiguousarray(indices, dtype=np.uint8).reshape(height, width)
     pal = np.ascontiguousarray(palette, dtype=np.uint32).ravel()
+    if pal.size == 0 or pal.size > 256:
+        raise ValueError("palette must hold 1..256 colours")
+    if idx.size and int(idx.max()) >= pal.size:
+        raise ValueError("an index is past the end of the palette")
     plte = np.stack([(pal >> 16) & 0xFF, (pal >> 8) & 0xFF, pal & 0xFF], axis=1).astype(np.uint8).tobytes()
     alpha = ((pal >> 24) & 0xFF).astype(np.uint8)
     raw = np.concatenate([np.zeros((height, 1), np.uint8), idx], axis=1).tobytes()   # filter type 0 on every row

@@ -100,6 +100,32 @@ class Context:
                                                      int(bool(dither)), _p(sd), ctypes.c_void_p(out_ptr), _p(palettes), _p(palette_lens),
                                                      _p(has_alpha)))
 
+    def convert_indexed(self, kind, images, n_max_colors, dither, seeds=None, with_argb=False):
+        """nq_convert_ragged_indexed: the palette index of every output pixel, computed on the GPU (the lowest index of the
+        pixel's colour, include/nquant_b200.h). images: list of (height, width) uint32 host arrays. Returns (list of
+        (height, width) uint8 index maps, list of ARGB outputs or None unless with_argb, palettes (n, 256), palette_lens,
+        has_alpha)."""
+        R = _Ragged(images, argb_out=with_argb)
+        idx = [np.empty(im.shape, dtype=np.uint8) for im in R.ins]
+        idx_ptrs = (ctypes.c_void_p * R.n)(*[a.ctypes.data for a in idx])
+        sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._check(self._L.nq_convert_ragged_indexed(self._h, kind, R.in_ptrs, _p(R.widths), _p(R.heights), R.n, int(n_max_colors),
+                                                      int(bool(dither)), _p(sd), idx_ptrs, R.out_ptrs, _p(R.pal), _p(R.plen), _p(R.ha)))
+        return idx, R.outs, R.pal, R.plen, R.ha
+
+    def convert_indexed_ptr(self, kind, in_ptr, index_ptr, widths, heights, n_max_colors, dither, seeds=None, out_ptr=None,
+                            palettes=None, palette_lens=None, has_alpha=None):
+        """nq_convert_ragged_indexed_device: device buffers (e.g. torch tensors), images packed back to back; the index map
+        of image i starts at byte sum_{j<i} widths[j]*heights[j] of index_ptr. out_ptr (optional) receives the ARGB output.
+        Every pointer 16-byte aligned. palettes / palette_lens / has_alpha: optional host arrays that receive the results."""
+        w = np.ascontiguousarray(widths, dtype=np.int32)
+        h = np.ascontiguousarray(heights, dtype=np.int32)
+        sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._check(self._L.nq_convert_ragged_indexed_device(self._h, kind, ctypes.c_void_p(in_ptr), _p(w), _p(h), len(w), int(n_max_colors),
+                                                             int(bool(dither)), _p(sd), ctypes.c_void_p(index_ptr),
+                                                             ctypes.c_void_p(out_ptr) if out_ptr else None, _p(palettes), _p(palette_lens),
+                                                             _p(has_alpha)))
+
     def dither_with_palette(self, kind, argb, width, height, n_max_colors, dither, palette, seed=0):
         argb = np.ascontiguousarray(argb, dtype=np.uint32)
         palette = np.ascontiguousarray(palette, dtype=np.uint32)
@@ -236,16 +262,18 @@ def convert_batch_multi(contexts, kind, argb, width, height, n_max_colors, dithe
 class _Ragged:
     """Host arguments of the ragged entry points: sides, per-image pointer arrays, result arrays."""
 
-    def __init__(self, images):
+    def __init__(self, images, argb_out=True):
         self.ins = [np.ascontiguousarray(im, dtype=np.uint32) for im in images]
         if any(im.ndim != 2 for im in self.ins):
             raise NQuantError(_lib.NQ_ERR_ARG, "every image must be a (height, width) array")
         self.n = len(self.ins)
         self.heights = np.array([im.shape[0] for im in self.ins], dtype=np.int32)
         self.widths = np.array([im.shape[1] for im in self.ins], dtype=np.int32)
-        self.outs = [np.empty_like(im) for im in self.ins]
         self.in_ptrs = (ctypes.c_void_p * self.n)(*[im.ctypes.data for im in self.ins])
-        self.out_ptrs = (ctypes.c_void_p * self.n)(*[o.ctypes.data for o in self.outs])
+        self.outs, self.out_ptrs = None, None
+        if argb_out:
+            self.outs = [np.empty_like(im) for im in self.ins]
+            self.out_ptrs = (ctypes.c_void_p * self.n)(*[o.ctypes.data for o in self.outs])
         self.pal = np.zeros((self.n, 256), dtype=np.uint32)
         self.plen = np.zeros(self.n, dtype=np.int32)
         self.ha = np.zeros(self.n, dtype=np.int32)
@@ -307,6 +335,17 @@ class PnnQuantizer:
         self._has_alpha = bool(ha[0])
         self.info = ctx.image_info(0)
         return out[0]
+
+    def convert_indexed(self, nMaxColors, dither):
+        """convert() as palette indices: one uint8 per pixel, palette[index] is the colour convert() returns (the lowest
+        index of that colour). Sets palette, hasAlpha() and info like convert()."""
+        ctx = default_context(self.device)
+        idx, _, pal, plen, ha = ctx.convert_indexed(self.KIND, [self.pixels.reshape(self.height, self.width)], nMaxColors, dither,
+                                                    seeds=[self.rng_seed])
+        self.palette = pal[0, :plen[0]].copy()
+        self._has_alpha = bool(ha[0])
+        self.info = ctx.image_info(0)
+        return idx[0].reshape(-1)
 
     def hasAlpha(self):
         """boolean hasAlpha() (PnnQuantizer.java:458)."""
