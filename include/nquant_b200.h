@@ -147,6 +147,35 @@ int nq_convert_ragged_indexed_device(nq_ctx* ctx, int kind, const uint32_t* d_ar
                                      int n_images, int n_max_colors, int dither, const uint64_t* rng_seeds, uint8_t* d_index_out,
                                      uint32_t* d_argb_out, uint32_t* palettes_out, int* palette_lens, int* has_alpha);
 
+/* REMAP: dither images to palettes the caller already has (one palette for the frames of an animation, a fixed hardware or
+ * e-ink palette, a palette computed once and reused) -- convert() with the palette replaced, without the merge loop.
+ * Image i goes through convert(n_max_colors, dither) (PnnQuantizer.java:409-456) as far as the palette: the alpha scan,
+ * and the histogram only as far as it feeds the scalars of pnnquan (maxbins, weight, the PR/PG/PB/PA reset, quan_rt,
+ * isNano, ratio with its re-tune, the few-colours return of PnnLABQuantizer.java:193-206), or the fixed-palette branch for
+ * n_max_colors <= 2. Then the caller's palette takes the place of pnnquan's (or of the fixed one) and the dither runs as
+ * convert runs it (PnnQuantizer.java:393-407, PnnLABQuantizer.java:492-522), BlueNoise pass, pixelMap.size() weight and
+ * seeded draws included. So remapping an image to the palette convert gave it, with the same n_max_colors and seed,
+ * returns convert's output bit for bit. Decisions the reference keys on the palette length (the BlueNoise pass for more
+ * than 32 entries, the closest-colour rules) follow the caller's palette; those keyed on nMaxColors (the histogram key
+ * layout, weight, the saliency of pnnquan) follow n_max_colors. The two may differ.
+ * palettes_in: HOST memory, n_palettes x 256 entries (palette p at p*256); palette_lens_in: n_palettes lengths, each
+ * 1..256; n_palettes is 1 (one palette for every image) or n_images. argb_out and index_out are each optional, but not
+ * both NULL; index_out[i] receives the LOWEST palette index of each output pixel's colour, as in
+ * nq_convert_ragged_indexed, so palettes with duplicate entries are well defined. The merge loop never runs, so
+ * NQ_ERR_COLOR cannot occur and nq_get_image_info reports merges == 0. PnnLABQuantizer with dither == 0,
+ * semi-transparent pixels and a palette of more than 32 entries returns NQ_ERR_UNSUPPORTED, as convert does. Sizes,
+ * seeds, has_alpha, streams, chunking and the other errors are as in nq_convert_ragged; bad palette arguments return
+ * NQ_ERR_ARG before any work starts. */
+int nq_remap_ragged(nq_ctx* ctx, int kind, const uint32_t* const* argb_in, const int* widths, const int* heights, int n_images,
+                    int n_max_colors, const uint32_t* palettes_in, const int* palette_lens_in, int n_palettes, int dither,
+                    const uint64_t* rng_seeds, uint32_t* const* argb_out, uint8_t* const* index_out, int* has_alpha);
+
+/* The same with DEVICE buffers packed as in nq_convert_ragged_indexed_device (every device base pointer 16-byte aligned);
+ * palettes_in and palette_lens_in stay host memory. d_argb_out NULL: the colours go to scratch memory of the context. */
+int nq_remap_ragged_device(nq_ctx* ctx, int kind, const uint32_t* d_argb_in, const int* widths, const int* heights, int n_images,
+                           int n_max_colors, const uint32_t* palettes_in, const int* palette_lens_in, int n_palettes, int dither,
+                           const uint64_t* rng_seeds, uint32_t* d_argb_out, uint8_t* d_index_out, int* has_alpha);
+
 /* nq_convert_ragged over several contexts with the dynamic queue of nq_convert_batch_multi (pieces of queue_images
  * images, 0 = one piece per context). */
 int nq_convert_ragged_multi(nq_ctx** contexts, int n_contexts, int kind, const uint32_t* const* argb_in, const int* widths,
@@ -156,7 +185,8 @@ int nq_convert_ragged_multi(nq_ctx** contexts, int n_contexts, int kind, const u
 /* Stage hook (parity + profiling): GilbertCurve.dither / BlueNoise.dither with a caller-supplied
  * palette (PnnQuantizer.java:393-407, PnnLABQuantizer.java:492-522). Runs the alpha scan and the
  * histogram-derived scalars as convert() would, but replaces the palette pnnquan produced by
- * palette_in before dithering. Host buffers. */
+ * palette_in before dithering. Host buffers. For n_max_colors > 2 this is nq_remap_ragged of one image; for
+ * n_max_colors <= 2 the image is dithered to the fixed palette of PnnQuantizer.java:441-452 and palette_in is not used. */
 int nq_dither_with_palette(nq_ctx* ctx, int kind, const uint32_t* argb_in, int width, int height, int n_max_colors,
                            int dither, uint64_t rng_seed, const uint32_t* palette_in, int palette_len, uint32_t* argb_out);
 

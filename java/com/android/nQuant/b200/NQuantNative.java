@@ -52,6 +52,10 @@ final class NQuantNative {
 	//                               index_out[], argb_out[] (NULL: colours not returned), palettes_out, palette_lens, has_alpha)
 	static final MethodHandle nq_convert_ragged_indexed = h("nq_convert_ragged_indexed",
 		FunctionDescriptor.of(I, P, I, P, P, P, I, I, I, P, P, P, P, P, P));
+	// int nq_remap_ragged(ctx, kind, argb_in[], widths, heights, n_images, n_max_colors, palettes_in, palette_lens_in, n_palettes,
+	//                     dither, rng_seeds, argb_out[] (or NULL), index_out[] (or NULL), has_alpha): dither to the caller's palettes
+	static final MethodHandle nq_remap_ragged = h("nq_remap_ragged",
+		FunctionDescriptor.of(I, P, I, P, P, P, I, I, P, P, I, I, P, P, P, P));
 	// int nq_device_count(void)
 	static final MethodHandle nq_device_count = h("nq_device_count", FunctionDescriptor.of(I));
 	// int nq_set_spec_dither(ctx, on, segment, warmup): speculative segment-parallel error diffusion, on by default (DESIGN.md 7.1)

@@ -106,6 +106,44 @@ public class PnnQuantizer implements AutoCloseable {
 		}
 	}
 
+	/**
+	 * convert() with the palette replaced by the caller's (nq_remap_ragged): the alpha scan and the histogram's scalars as
+	 * convert(nMaxColors, dither) computes them, no merge loop, then the dither to {@code palette} (1..256 colours). Remapping
+	 * to the palette convert() returned, with the same nMaxColors and seed, returns convert()'s output. Sets hasAlpha() and
+	 * makes getPalette() return {@code palette}.
+	 */
+	public int[] remap(int[] palette, int nMaxColors, boolean dither) throws Exception {
+		if (palette.length < 1 || palette.length > 256)
+			throw new IllegalArgumentException("palette must hold 1..256 colours");
+		try (Arena arena = Arena.ofConfined()) {
+			final long n = (long) width * height;
+			MemorySegment in = arena.allocate(ValueLayout.ADDRESS);
+			in.set(ValueLayout.ADDRESS, 0, arena.allocateFrom(ValueLayout.JAVA_INT, pixels));
+			MemorySegment out = arena.allocate(ValueLayout.JAVA_INT, n);
+			MemorySegment outs = arena.allocate(ValueLayout.ADDRESS);
+			outs.set(ValueLayout.ADDRESS, 0, out);
+			MemorySegment w = arena.allocateFrom(ValueLayout.JAVA_INT, width);
+			MemorySegment h = arena.allocateFrom(ValueLayout.JAVA_INT, height);
+			MemorySegment seed = arena.allocateFrom(ValueLayout.JAVA_LONG, rngSeed);
+			MemorySegment pal = arena.allocate(ValueLayout.JAVA_INT, 256);
+			MemorySegment.copy(palette, 0, pal, ValueLayout.JAVA_INT, 0, palette.length);
+			MemorySegment plen = arena.allocateFrom(ValueLayout.JAVA_INT, palette.length);
+			MemorySegment alpha = arena.allocate(ValueLayout.JAVA_INT);
+			int rc;
+			try {
+				rc = (int) NQuantNative.nq_remap_ragged.invokeExact(NQuantNative.context(device), kind(), in, w, h, 1, nMaxColors, pal, plen, 1,
+					dither ? 1 : 0, seed, outs, MemorySegment.NULL, alpha);
+			} catch (Throwable t) {
+				throw new Exception(t);
+			}
+			if (rc != 0)
+				throw new Exception("nq_remap_ragged failed (" + rc + "): " + NQuantNative.lastError());
+			hasAlpha = alpha.get(ValueLayout.JAVA_INT, 0) != 0;
+			this.palette = palette.clone();
+			return out.toArray(ValueLayout.JAVA_INT);
+		}
+	}
+
 	/** boolean hasAlpha() (PnnQuantizer.java:458). */
 	public boolean hasAlpha() {
 		return hasAlpha;

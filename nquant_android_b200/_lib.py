@@ -14,7 +14,7 @@ SYMBOLS = [
     "nq_synth_device", "nq_get_stage_times", "nq_set_stream", "nq_debug_ciede", "nq_sizeof_image_info",
     "nq_set_spec_dither", "nq_get_spec_stats", "nq_reset_stream", "nq_set_chunk_images", "nq_get_kernel_times", "nq_convert_batch_multi", "nq_histogram",
     "nq_convert_ragged", "nq_convert_ragged_device", "nq_convert_ragged_multi",
-    "nq_convert_ragged_indexed", "nq_convert_ragged_indexed_device",
+    "nq_convert_ragged_indexed", "nq_convert_ragged_indexed_device", "nq_remap_ragged", "nq_remap_ragged_device",
 ]
 
 NQ_KIND_PNN, NQ_KIND_PNNLAB = 0, 1
@@ -72,6 +72,8 @@ def load():
     L.nq_convert_ragged_device.argtypes = [vp, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp]
     L.nq_convert_ragged_indexed.argtypes = [vp, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, vp]
     L.nq_convert_ragged_indexed_device.argtypes = [vp, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, vp]
+    L.nq_remap_ragged.argtypes = [vp, ci, vp, vp, vp, ci, ci, vp, vp, ci, ci, vp, vp, vp, vp]
+    L.nq_remap_ragged_device.argtypes = [vp, ci, vp, vp, vp, ci, ci, vp, vp, ci, ci, vp, vp, vp, vp]
     L.nq_convert_ragged_multi.argtypes = [vp, ci, ci, vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, ci]
     L.nq_dither_with_palette.argtypes = [vp, ci, vp, ci, ci, ci, ci, u64, vp, ci, vp]
     L.nq_gilbert_order.argtypes = [ci, ci, vp]

@@ -171,9 +171,15 @@ __global__ void k_ciede_probe(const float* l1, const float* l2, float* out, int*
   out[4 * i] = tL; out[4 * i + 1] = tC; out[4 * i + 2] = tH; out[4 * i + 3] = tRT;
 }
 
-__global__ void k_set_palette(NqImage* imgs, int img, const uint32_t* pal, int plen) {
-  if (threadIdx.x < plen) imgs[img].palette[threadIdx.x] = pal[threadIdx.x];
-  if (threadIdx.x == 0) imgs[img].paletteLen = plen;
+// ---- palettes of a remap call (nq_remap_ragged*): one CTA per image of the chunk, before its k_dither_setup ------------
+// Palette p is at pal + p * NQ_MAXK with len[p] entries; image i takes palette i * perImage (0: one palette for all). No
+// merge loop ran, so the image reports no merges.
+__global__ void k_install_palettes(NqImage* imgs, const uint32_t* pal, const int* len, int perImage) {
+  NqImage& I = imgs[blockIdx.x];
+  const size_t p = (size_t)blockIdx.x * perImage;
+  const int plen = len[p];
+  for (int k = threadIdx.x; k < plen; k += blockDim.x) I.palette[k] = pal[p * NQ_MAXK + k];
+  if (threadIdx.x == 0) { I.paletteLen = plen; I.callerPalette = 1; I.extbins = 0; }
 }
 
 // one RGB->Lab table per device, shared by every context on it
@@ -234,6 +240,8 @@ struct nq_ctx {
   uint32_t* dIn = nullptr;
   uint32_t* dOut = nullptr;
   size_t inBytes = 0, outBytes = 0;
+  uint32_t* dPal = nullptr;           // the palettes and their lengths of a remap call (upload_palettes)
+  size_t palBytes = 0;
   // per-stage device timing (CUDA events on the internal streams, summed over the chunks of a call)
   double stageMs[NQ_NSTAGES] = {};
   unsigned long long stageLaunches[NQ_NSTAGES] = {};
@@ -444,6 +452,10 @@ struct NvtxRange {
   ~NvtxRange() { nvtxRangePop(); }
 };
 
+// The palettes of a remap call, on the device: palette p at pal + p * NQ_MAXK with len[p] entries; image i of the call takes
+// palette i * perImage (perImage 0: one palette shared by the call). maxLen: the longest.
+struct RemapPalettes { const uint32_t* pal; const int* len; int perImage, maxLen; };
+
 // Images [0, n) of a group, every one with its own geometry; the per-image pointers start at the group's first image.
 // Pixels are packed back to back in the call's device buffers: image i at dIn + off[i], off[i + 1] - off[i] pixels.
 struct GroupArgs {
@@ -453,11 +465,15 @@ struct GroupArgs {
   const size_t* off;                // n + 1 entries
   const uint32_t* const* order;     // Gilbert table of each image's size (nullptr with stopAfterSweep)
   const uint64_t* seeds;
-  const uint32_t* dPalIn;
-  int palInLen;
   const uint32_t* const* hIn;       // host pixels of each image (nullptr: dIn is the caller's device buffer and already holds them)
   uint32_t* const* hOut;            // (nullptr: no host copy of the colours)
   bool stopAfterSweep = false;      // stage hook nq_histogram: no merge loop, no dither
+  // remap calls: the callers' palettes on the device (see k_install_palettes), nullptr in convert calls. The front stops
+  // after the scalars of pnnquan (no find_nn sweep, no merge loop) and the palettes are installed before the dither.
+  const uint32_t* dPal = nullptr;
+  const int* dPalLen = nullptr;
+  int palPerImage = 0;
+  int palMax = 0;                   // longest palette of the call (convert: nmax): gates the BlueNoise pass kernels
   // index-map calls: the call's packed index plane, image i at byte off[i] (nullptr: no index map), and the host
   // destination of each image's indices (nullptr: the plane is the caller's device buffer)
   unsigned char* dIdx = nullptr;
@@ -724,25 +740,28 @@ int enqueue_front(nq_ctx* c, Chunk& ch, const GroupArgs& A, const uint32_t* dIn,
     } else {
       const int nruns = (npix + NQ_RUN - 1) / NQ_RUN;
       nq::k_lab_count<<<pg, 256, 0, st>>>(dI, dS); ++c->launches;
-      nq::k_lab_scan_keys<<<n, 1024, 0, st>>>(dI, dS); ++c->launches;
-      for (int g0 = 0; g0 < n; g0 += c->sortSets) {   // images of one group own distinct sort scratch sets
-        const int gn = std::min(c->sortSets, n - g0);
-        NqImage* gi = dI + g0;
-        NqSlot* gs = dS + g0;
-        const dim3 rg(std::max(1, std::min((nruns + 7) / 8, std::max(1, c->smCount * 8 / gn))), gn);
-        nq::k_radix_count<0><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
-        nq::k_radix_offsets<<<gn, 256, 0, st>>>(gi, gs); ++c->launches;
-        nq::k_radix_scatter<0><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
-        nq::k_radix_count<1><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
-        nq::k_radix_offsets<<<gn, 256, 0, st>>>(gi, gs); ++c->launches;
-        nq::k_radix_scatter<1><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
-        const dim3 bg(std::max(1, c->smCount * 8 / gn), gn);
-        nq::k_lab_bin_sum<<<bg, 256, 0, st>>>(gi, gs); ++c->launches;
+      if (!A.dPal) {   // the bin sums in strict pixel order; a remap needs the key counts alone
+        nq::k_lab_scan_keys<<<n, 1024, 0, st>>>(dI, dS); ++c->launches;
+        for (int g0 = 0; g0 < n; g0 += c->sortSets) {   // images of one group own distinct sort scratch sets
+          const int gn = std::min(c->sortSets, n - g0);
+          NqImage* gi = dI + g0;
+          NqSlot* gs = dS + g0;
+          const dim3 rg(std::max(1, std::min((nruns + 7) / 8, std::max(1, c->smCount * 8 / gn))), gn);
+          nq::k_radix_count<0><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
+          nq::k_radix_offsets<<<gn, 256, 0, st>>>(gi, gs); ++c->launches;
+          nq::k_radix_scatter<0><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
+          nq::k_radix_count<1><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
+          nq::k_radix_offsets<<<gn, 256, 0, st>>>(gi, gs); ++c->launches;
+          nq::k_radix_scatter<1><<<rg, 256, 0, st>>>(gi, gs); ++c->launches;
+          const dim3 bg(std::max(1, c->smCount * 8 / gn), gn);
+          nq::k_lab_bin_sum<<<bg, 256, 0, st>>>(gi, gs); ++c->launches;
+        }
       }
-      nq::k_finalize_lab<<<n, 1024, 0, st>>>(dI, dS); ++c->launches;
-      nq::k_lab_fewcolors<<<n, 256, 0, st>>>(dI, dS); ++c->launches;
+      nq::k_finalize_lab<<<n, 1024, 0, st>>>(dI, dS, A.dPal ? 0 : 1); ++c->launches;   // a remap needs the scalars only
+      nq::k_lab_fewcolors<<<n, 256, 0, st>>>(dI, dS); ++c->launches;   // ratio of the few-colours return (PL:193-206)
     }
     mark(2);
+    if (A.dPal) { mark(3); mark(4); CU(cudaGetLastError()); return NQ_OK; }   // remap: no find_nn sweep, no merge loop
     if (kind == NQ_KIND_RGB) {
       nq::k_rgb_blocks<<<dim3(2, n), 256, 0, st>>>(dI, dS); ++c->launches;
       nq::k_find_nn_all<<<c->smCount * 8, 256, 0, st>>>(dI, dS, n); ++c->launches;
@@ -808,11 +827,11 @@ int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A) {
   unsigned long long l0 = c->launches;
   CU(cudaStreamWaitEvent(st, ch.ev[4], 0));
   CU(cudaEventRecord(ch.evD[0], st));
-  nq::k_dither_setup<<<(n + 63) / 64, 64, 0, st>>>(dI, dS, n); ++c->launches;
-  if (A.dPalIn) {
-    for (int i = 0; i < n; ++i) { k_set_palette<<<1, 256, 0, st>>>(dI, i, A.dPalIn, A.palInLen); ++c->launches; }
-    nq::k_dither_setup<<<(n + 63) / 64, 64, 0, st>>>(dI, dS, n); ++c->launches;
+  if (A.dPal) {
+    const size_t p0 = (size_t)ch.base * A.palPerImage;
+    k_install_palettes<<<n, 256, 0, st>>>(dI, A.dPal + p0 * NQ_MAXK, A.dPalLen + p0, A.palPerImage); ++c->launches;
   }
+  nq::k_dither_setup<<<(n + 63) / 64, 64, 0, st>>>(dI, dS, n); ++c->launches;
   const dim3 pg(pixel_grid_x(c, npix, n), n);
   if (kind == NQ_KIND_LAB && c->debug) { nq::k_saliency<<<pg, 256, 0, st>>>(dI, dS); ++c->launches; }
   if (kind == NQ_KIND_LAB) { nq::k_build_cells<<<dim3(std::max(1, std::min(128, c->smCount * 8 / n)), n), 256, 0, st>>>(dI, dS); ++c->launches; }
@@ -839,7 +858,7 @@ int run_dither(nq_ctx* c, Chunk& ch, const GroupArgs& A) {
   cudaEventRecord(ch.evK[4], ax);
   nq::k_dither_sorted<<<n, 32, 0, ax>>>(dI, dS); ++c->launches;
   cudaEventRecord(ch.evK[5], ax);
-  if (kind == NQ_KIND_RGB && !A.dither && A.nmax > 32) {   // BlueNoise.dither second pass, one thread per pixel (images flagged bnParallel)
+  if (kind == NQ_KIND_RGB && !A.dither && A.palMax > 32) {   // BlueNoise.dither second pass, one thread per pixel (images flagged bnParallel)
     nq::k_bn_rgb_init<<<dim3(8, n), 256, 0, ax>>>(dI, dS); ++c->launches;
     nq::k_bn_rgb_a<<<pg, 256, 0, ax>>>(dI, dS); ++c->launches;
     nq::k_bn_rgb_b<<<dim3(16, n), 256, 0, ax>>>(dI, dS); ++c->launches;
@@ -1015,18 +1034,22 @@ int convert_group(nq_ctx* c, const GroupArgs& A, int n, const uint32_t* dIn, uin
 // the whole call, the images packed back to back. hIn / hOut (optional): one host pointer per image, read from / written to
 // chunk by chunk, overlapped with the kernels. The workspace is sized by the largest image of the call. dIdx (optional): the
 // index plane, image i at byte off[i], filled by k_index_map; hIdx (optional): one host pointer per image it is copied to.
+// remap (optional): the call's palettes on the device, see RemapPalettes.
 int convert_device(nq_ctx* c, int kind, int n, const int* ws, const int* hs, const uint32_t* dIn, uint32_t* dOut, int nmax, int dither,
-                   const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn, int palInLen,
+                   const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const RemapPalettes* remap,
                    const uint32_t* const* hIn = nullptr, uint32_t* const* hOut = nullptr, bool stopAfterSweep = false,
                    unsigned char* dIdx = nullptr, uint8_t* const* hIdx = nullptr) {
   CU(cudaSetDevice(c->device));
   std::vector<size_t> off(n + 1, 0);
   int npix = 1;
   for (int i = 0; i < n; ++i) { off[i + 1] = off[i] + (size_t)ws[i] * hs[i]; npix = std::max(npix, ws[i] * hs[i]); }
+  // The BlueNoise second pass runs for palettes of more than 32 entries (PQ:403, PL:515): convert's palette has at most
+  // nmax, a remap's the length the caller gave, which may be on the other side of 32.
+  const int palMax = remap ? remap->maxLen : nmax;
   // the BlueNoise second pass of PnnLABQuantizer weighs by pixelMap.size() (PL:511-513): track it only then
-  const bool needBits = kind == NQ_KIND_LAB && !dither && nmax > 32;
+  const bool needBits = kind == NQ_KIND_LAB && !dither && palMax > 32;
   // PnnQuantizer's BlueNoise second pass runs one thread per pixel and keeps the first-pass indices next to the output
-  const bool needIdx = kind == NQ_KIND_RGB && !dither && nmax > 32;
+  const bool needIdx = kind == NQ_KIND_RGB && !dither && palMax > 32;
   int rc = ensure_workspace(c, kind, npix, n, needBits, needIdx);
   if (rc) return rc;
   std::vector<const uint32_t*> order;
@@ -1038,8 +1061,13 @@ int convert_device(nq_ctx* c, int kind, int n, const int* ws, const int* hs, con
   for (int base = 0; base < n; base += c->wsSlots) {
     const int m = std::min(c->wsSlots, n - base);
     GroupArgs A{kind, nmax, dither, ws + base, hs + base, off.data() + base, order.empty() ? nullptr : order.data() + base,
-                seeds ? seeds + base : nullptr, dPalIn, palInLen, hIn ? hIn + base : nullptr, hOut ? hOut + base : nullptr};
+                seeds ? seeds + base : nullptr, hIn ? hIn + base : nullptr, hOut ? hOut + base : nullptr};
     A.stopAfterSweep = stopAfterSweep;
+    A.palMax = palMax;
+    if (remap) {
+      const size_t p0 = (size_t)base * remap->perImage;
+      A.dPal = remap->pal + p0 * NQ_MAXK; A.dPalLen = remap->len + p0; A.palPerImage = remap->perImage;
+    }
     A.dIdx = dIdx;
     A.hIdx = hIdx ? hIdx + base : nullptr;
     rc = convert_group(c, A, m, dIn, dOut, base);
@@ -1076,14 +1104,14 @@ int ensure_stage(nq_ctx* c, size_t bytes) {
 // complete (after the chunk's dither, or for the complete prefix the progressive copy-out hands on), so no kernel reads
 // that input again. Later images' input starts at byte 4 * off[i+1] or later and stays intact.
 int convert_host(nq_ctx* c, int kind, int n, const int* ws, const int* hs, const uint32_t* const* in, uint32_t* const* out, int nmax,
-                 int dither, const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const uint32_t* dPalIn = nullptr,
-                 int palInLen = 0, bool stopAfterSweep = false, uint8_t* const* idx = nullptr) {
+                 int dither, const uint64_t* seeds, uint32_t* palettes, int* plens, int* hasAlpha, const RemapPalettes* remap = nullptr,
+                 bool stopAfterSweep = false, uint8_t* const* idx = nullptr) {
   CU(cudaSetDevice(c->device));
   size_t total = 0;
   for (int i = 0; i < n; ++i) total += (size_t)ws[i] * hs[i];
   int rc = ensure_stage(c, total * 4);
   if (rc) return rc;
-  rc = convert_device(c, kind, n, ws, hs, c->dIn, c->dOut, nmax, dither, seeds, palettes, plens, hasAlpha, dPalIn, palInLen, in, out, stopAfterSweep,
+  rc = convert_device(c, kind, n, ws, hs, c->dIn, c->dOut, nmax, dither, seeds, palettes, plens, hasAlpha, remap, in, out, stopAfterSweep,
                       idx ? reinterpret_cast<unsigned char*>(c->dIn) : nullptr, idx);
   if (rc) return rc;
   CU(cudaStreamSynchronize(c->stream));
@@ -1120,6 +1148,7 @@ void destroy_ctx(nq_ctx* c, bool dropLut) {
   if (c->ws) cudaFree(c->ws);
   if (c->dIn) cudaFree(c->dIn);
   if (c->dOut) cudaFree(c->dOut);
+  if (c->dPal) cudaFree(c->dPal);
   if (c->dSpec) cudaFree(c->dSpec);
   if (c->specBuf) cudaFree(c->specBuf);
   if (c->dSpecPool) cudaFree(c->dSpecPool);
@@ -1181,6 +1210,28 @@ int run_multi(nq_ctx** ctxs, int nctx, int n, int queueImages, Convert convert) 
   worker(0);
   for (auto& t : threads) t.join();
   if (firstRc.load() != NQ_OK) return fail(firstRc.load(), errMsg);
+  return NQ_OK;
+}
+// The palette arguments of a remap call, checked before any work starts.
+int check_palettes(int n, const uint32_t* pals, const int* lens, int nPal) {
+  if (!pals || !lens) return fail(NQ_ERR_ARG, "null palettes or palette lengths");
+  if (nPal != 1 && nPal != n) return fail(NQ_ERR_ARG, "n_palettes must be 1 or n_images");
+  for (int p = 0; p < nPal; ++p)
+    if (lens[p] < 1 || lens[p] > NQ_MAXK) return fail(NQ_ERR_ARG, "palette " + std::to_string(p) + ": length must be 1..256");
+  return NQ_OK;
+}
+// One copy of the palettes (NQ_MAXK entries each) and their lengths to the context's palette buffer, ordered before the
+// call's work on the context's stream.
+int upload_palettes(nq_ctx* c, int n, const uint32_t* pals, const int* lens, int nPal, RemapPalettes* R) {
+  CU(cudaSetDevice(c->device));
+  const size_t palBytes = (size_t)nPal * NQ_MAXK * 4;
+  int rc = ensure_buffer(&c->dPal, &c->palBytes, palBytes + (size_t)nPal * 4);
+  if (rc) return rc;
+  int* dLen = reinterpret_cast<int*>(c->dPal + (size_t)nPal * NQ_MAXK);
+  CU(cudaMemcpyAsync(c->dPal, pals, palBytes, cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(dLen, lens, (size_t)nPal * 4, cudaMemcpyHostToDevice, c->stream));
+  R->pal = c->dPal; R->len = dLen; R->perImage = nPal == n ? 1 : 0;
+  R->maxLen = *std::max_element(lens, lens + nPal);
   return NQ_OK;
 }
 int check_contexts(nq_ctx** ctxs, int nctx, int queueImages) {
@@ -1282,7 +1333,7 @@ int nq_convert_batch_device(nq_ctx* c, int kind, const uint32_t* d_in, int n, in
   if (rc) return rc;
   NvtxRange nv("nq_convert_batch_device");
   UniformBatch B(n, w, h);
-  return convert_device(c, kind, n, B.w.data(), B.h.data(), d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0);
+  return convert_device(c, kind, n, B.w.data(), B.h.data(), d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr);
 }
 
 int nq_convert_ragged_device(nq_ctx* c, int kind, const uint32_t* d_in, const int* ws, const int* hs, int n, int nmax, int dither,
@@ -1290,7 +1341,7 @@ int nq_convert_ragged_device(nq_ctx* c, int kind, const uint32_t* d_in, const in
   int rc = check_ragged(c, kind, d_in, ws, hs, n, nmax, d_out);
   if (rc) return rc;
   NvtxRange nv("nq_convert_ragged_device");
-  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0);
+  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr);
 }
 
 int nq_convert_batch(nq_ctx* c, int kind, const uint32_t* in, int n, int w, int h, int nmax, int dither, const uint64_t* seeds,
@@ -1318,7 +1369,7 @@ int nq_convert_ragged_indexed(nq_ctx* c, int kind, const uint32_t* const* in, co
   for (int i = 0; i < n; ++i)
     if (!idx[i]) return fail(NQ_ERR_ARG, "image " + std::to_string(i) + ": null index buffer");
   NvtxRange nv("nq_convert_ragged_indexed");
-  return convert_host(c, kind, n, ws, hs, in, out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0, false, idx);
+  return convert_host(c, kind, n, ws, hs, in, out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, false, idx);
 }
 
 int nq_convert_ragged_indexed_device(nq_ctx* c, int kind, const uint32_t* d_in, const int* ws, const int* hs, int n, int nmax, int dither,
@@ -1334,7 +1385,7 @@ int nq_convert_ragged_indexed_device(nq_ctx* c, int kind, const uint32_t* d_in, 
     if ((rc = ensure_buffer(&c->dOut, &c->outBytes, total * 4))) return rc;
     d_out = c->dOut;
   }
-  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, 0, nullptr, nullptr, false, d_idx);
+  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, palettes, plens, hasAlpha, nullptr, nullptr, nullptr, false, d_idx);
 }
 
 int nq_convert_batch_multi(nq_ctx** ctxs, int nctx, int kind, const uint32_t* in, int n, int w, int h, int nmax, int dither,
@@ -1368,16 +1419,52 @@ int nq_convert(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax, 
   return nq_convert_batch(c, kind, in, 1, w, h, nmax, dither, &seed, out, palette, plen, hasAlpha);
 }
 
+int nq_remap_ragged(nq_ctx* c, int kind, const uint32_t* const* in, const int* ws, const int* hs, int n, int nmax,
+                    const uint32_t* pals, const int* plens, int nPal, int dither, const uint64_t* seeds, uint32_t* const* out,
+                    uint8_t* const* idx, int* hasAlpha) {
+  int rc = check_ragged(c, kind, in, ws, hs, n, nmax, in, in, out);
+  if (rc) return rc;
+  if (!out && !idx) return fail(NQ_ERR_ARG, "argb_out and index_out are both null");
+  for (int i = 0; idx && i < n; ++i)
+    if (!idx[i]) return fail(NQ_ERR_ARG, "image " + std::to_string(i) + ": null index buffer");
+  if ((rc = check_palettes(n, pals, plens, nPal))) return rc;
+  NvtxRange nv("nq_remap_ragged");
+  RemapPalettes R;
+  if ((rc = upload_palettes(c, n, pals, plens, nPal, &R))) return rc;
+  return convert_host(c, kind, n, ws, hs, in, out, nmax, dither, seeds, nullptr, nullptr, hasAlpha, &R, false, idx);
+}
+
+int nq_remap_ragged_device(nq_ctx* c, int kind, const uint32_t* d_in, const int* ws, const int* hs, int n, int nmax,
+                           const uint32_t* pals, const int* plens, int nPal, int dither, const uint64_t* seeds, uint32_t* d_out,
+                           uint8_t* d_idx, int* hasAlpha) {
+  int rc = check_ragged(c, kind, d_in, ws, hs, n, nmax, d_in);
+  if (rc) return rc;
+  if (!d_out && !d_idx) return fail(NQ_ERR_ARG, "d_argb_out and d_index_out are both null");
+  if (((uintptr_t)d_in | (uintptr_t)d_idx | (uintptr_t)d_out) & 15) return fail(NQ_ERR_ARG, "device buffers must be 16-byte aligned");
+  if ((rc = check_palettes(n, pals, plens, nPal))) return rc;
+  NvtxRange nv("nq_remap_ragged_device");
+  CU(cudaSetDevice(c->device));
+  if (!d_out) {   // the colours stay in the context's scratch
+    size_t total = 0;
+    for (int i = 0; i < n; ++i) total += (size_t)ws[i] * hs[i];
+    if ((rc = ensure_buffer(&c->dOut, &c->outBytes, total * 4))) return rc;
+    d_out = c->dOut;
+  }
+  RemapPalettes R;
+  if ((rc = upload_palettes(c, n, pals, plens, nPal, &R))) return rc;
+  return convert_device(c, kind, n, ws, hs, d_in, d_out, nmax, dither, seeds, nullptr, nullptr, hasAlpha, &R, nullptr, nullptr, false, d_idx);
+}
+
+// n_max_colors <= 2 dithers to the fixed palette, as this hook always has; above, it is a remap of one image.
 int nq_dither_with_palette(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax, int dither, uint64_t seed,
                            const uint32_t* palette, int plen, uint32_t* out) {
   int rc = check_args(c, kind, in, 1, w, h, nmax, out);
   if (rc) return rc;
   if (!palette || plen <= 0 || plen > NQ_MAXK) return fail(NQ_ERR_ARG, "palette_len must be 1..256");
-  CU(cudaSetDevice(c->device));
-  DevBuf dPal;
-  CU(dPal.alloc(NQ_MAXK * 4));
-  CU(cudaMemcpy(dPal.p, palette, (size_t)plen * 4, cudaMemcpyHostToDevice));
-  return convert_host(c, kind, 1, &w, &h, &in, &out, nmax, dither, &seed, nullptr, nullptr, nullptr, dPal.as<uint32_t>(), plen);
+  if (nmax <= 2) return convert_host(c, kind, 1, &w, &h, &in, &out, nmax, dither, &seed, nullptr, nullptr, nullptr);
+  std::vector<uint32_t> pal(NQ_MAXK, 0);
+  std::copy(palette, palette + plen, pal.begin());
+  return nq_remap_ragged(c, kind, &in, &w, &h, 1, nmax, pal.data(), &plen, 1, dither, &seed, &out, nullptr, nullptr);
 }
 
 int nq_histogram(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax, int* nBins, double* bins5, float* initErr, int* initNn, int capacity) {
@@ -1387,7 +1474,7 @@ int nq_histogram(nq_ctx* c, int kind, const uint32_t* in, int w, int h, int nmax
   const bool wasDebug = c->debug;
   c->debug = true;                                   // the hook returns what debug mode records after the find_nn sweep
   uint64_t seed = 0;
-  rc = convert_host(c, kind, 1, &w, &h, &in, nullptr, nmax, 1, &seed, nullptr, nullptr, nullptr, nullptr, 0, true);
+  rc = convert_host(c, kind, 1, &w, &h, &in, nullptr, nmax, 1, &seed, nullptr, nullptr, nullptr, nullptr, true);
   c->debug = wasDebug;
   if (rc) return rc;
   const DebugImage& D = c->dbg[0];

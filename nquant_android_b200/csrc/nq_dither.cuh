@@ -492,12 +492,14 @@ __global__ void k_dither_setup(NqImage* imgs, const NqSlot* slots, int nimg) {
   int img = blockIdx.x * blockDim.x + threadIdx.x;
   if (img >= nimg) return;
   NqImage& I = imgs[img];
-  if (I.nmax <= 2) {   // fixed palette (PQ:441-452)
+  if (I.nmax <= 2) {   // fixed palette (PQ:441-452); a caller's palette (remap) takes its place
     I.weight = 1;
-    I.paletteLen = I.nmax;
-    if (I.transIdx >= 0) { I.palette[0] = I.transColor; I.palette[1] = 0xFF000000u; }
-    else { I.palette[0] = 0xFF000000u; I.palette[1] = 0xFFFFFFFFu; }
-    if (I.nmax < 2) I.paletteLen = I.nmax < 0 ? 0 : I.nmax;
+    if (!I.callerPalette) {
+      I.paletteLen = I.nmax;
+      if (I.transIdx >= 0) { I.palette[0] = I.transColor; I.palette[1] = 0xFF000000u; }
+      else { I.palette[0] = 0xFF000000u; I.palette[1] = 0xFFFFFFFFu; }
+      if (I.nmax < 2) I.paletteLen = I.nmax < 0 ? 0 : I.nmax;
+    }
   }
   const int plen = I.paletteLen;
   const bool lab = I.kind == NQ_KIND_LAB;

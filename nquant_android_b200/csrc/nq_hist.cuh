@@ -485,7 +485,9 @@ __global__ void __launch_bounds__(256) k_lab_bin_sum(const NqImage* imgs, const 
 }
 
 // ---- compaction + means + pnnquan scalars, LAB (PL:160-241) --------------------------------------
-__global__ void __launch_bounds__(1024) k_finalize_lab(NqImage* imgs, const NqSlot* slots) {
+// means == 0 (remap front): the scalars alone, which depend on the key counts only (maxbins), so neither the sorted float
+// sums of k_lab_bin_sum nor the compacted bins are needed
+__global__ void __launch_bounds__(1024) k_finalize_lab(NqImage* imgs, const NqSlot* slots, int means) {
   __shared__ int sWarp[33];
   const int img = blockIdx.x;
   NqImage& I = imgs[img];
@@ -496,7 +498,7 @@ __global__ void __launch_bounds__(1024) k_finalize_lab(NqImage* imgs, const NqSl
   int c = 0;
   for (int k = 0; k < 64; ++k) c += S.hCnt[k0 + k] != 0;
   int total, j = block_excl_scan_1024(c, &total, sWarp);
-  for (int k = 0; k < 64; ++k) {
+  for (int k = 0; means && k < 64; ++k) {
     unsigned cnt = S.hCnt[k0 + k];
     if (!cnt) continue;
     float fc = cnt > 16777216u ? 16777216.f : (float)cnt;   // tb.cnt += 1.0f saturates at 2^24 (PL:154)
@@ -549,6 +551,7 @@ __global__ void __launch_bounds__(1024) k_finalize_lab(NqImage* imgs, const NqSl
     // pixelMap.size() <= nMaxColors needs maxbins <= nMaxColors: leave the decision to k_lab_fewcolors (PL:193-206)
     I.skipPnn = maxbins <= nmax ? 2 : 0;
   }
+  if (!means) return;
   __syncthreads();
   const int maxbins = I.maxbins, quan_rt = I.quan_rt, nmax = I.nmax;
   for (int b = t; b < maxbins; b += 1024) S.bCnt[b] = quan_lab(nmax, quan_rt, S.bCnt[b]);   // PL:210-217

@@ -49,6 +49,7 @@ struct NqImage {
                            // 3 handed back to k_dither_fifo
   unsigned int nonOpaque;  // pixels whose alpha is not 255 (alpha scan)
   int bnParallel;          // BlueNoise.dither second pass done by the per-pixel kernels k_bn_* instead of the serial warp
+  int callerPalette;       // the palette was installed by a remap call (k_install_palettes): k_dither_setup keeps it
   int pad1;
 };
 

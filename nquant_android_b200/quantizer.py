@@ -126,6 +126,39 @@ class Context:
                                                              ctypes.c_void_p(out_ptr) if out_ptr else None, _p(palettes), _p(palette_lens),
                                                              _p(has_alpha)))
 
+    def remap(self, kind, images, palettes, dither, n_max_colors=None, seeds=None, with_argb=True, with_indices=False):
+        """nq_remap_ragged: dither each image to a palette the caller already has, as convert() would with its palette
+        replaced, without the merge loop (include/nquant_b200.h). images: list of (height, width) uint32 host arrays.
+        palettes: one 1-D array of 1..256 colours shared by every image, or a list with one such array per image.
+        n_max_colors (the nMaxColors convert() would get) defaults to the longest palette, and at least 2. Returns (list of
+        ARGB outputs or None unless with_argb, list of uint8 index maps or None unless with_indices, has_alpha)."""
+        if not (with_argb or with_indices):
+            raise NQuantError(_lib.NQ_ERR_ARG, "with_argb and with_indices are both False")
+        R = _Ragged(images, argb_out=with_argb)
+        pal, plen, npal = _palettes(palettes, R.n)
+        nmax = max(2, int(plen.max())) if n_max_colors is None else int(n_max_colors)
+        idx, idx_ptrs = None, None
+        if with_indices:
+            idx = [np.empty(im.shape, dtype=np.uint8) for im in R.ins]
+            idx_ptrs = (ctypes.c_void_p * R.n)(*[a.ctypes.data for a in idx])
+        sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._check(self._L.nq_remap_ragged(self._h, kind, R.in_ptrs, _p(R.widths), _p(R.heights), R.n, nmax, _p(pal), _p(plen),
+                                            npal, int(bool(dither)), _p(sd), R.out_ptrs, idx_ptrs, _p(R.ha)))
+        return R.outs, idx, R.ha
+
+    def remap_ptr(self, kind, in_ptr, widths, heights, palettes, dither, n_max_colors=None, seeds=None, out_ptr=None, index_ptr=None,
+                  has_alpha=None):
+        """nq_remap_ragged_device: device buffers (e.g. torch tensors) packed as in convert_indexed_ptr, every pointer 16-byte
+        aligned; out_ptr and index_ptr are each optional, but not both. palettes and n_max_colors as in remap()."""
+        w = np.ascontiguousarray(widths, dtype=np.int32)
+        h = np.ascontiguousarray(heights, dtype=np.int32)
+        pal, plen, npal = _palettes(palettes, len(w))
+        nmax = max(2, int(plen.max())) if n_max_colors is None else int(n_max_colors)
+        sd = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._check(self._L.nq_remap_ragged_device(self._h, kind, ctypes.c_void_p(in_ptr), _p(w), _p(h), len(w), nmax, _p(pal), _p(plen),
+                                                   npal, int(bool(dither)), _p(sd), ctypes.c_void_p(out_ptr) if out_ptr else None,
+                                                   ctypes.c_void_p(index_ptr) if index_ptr else None, _p(has_alpha)))
+
     def dither_with_palette(self, kind, argb, width, height, n_max_colors, dither, palette, seed=0):
         argb = np.ascontiguousarray(argb, dtype=np.uint32)
         palette = np.ascontiguousarray(palette, dtype=np.uint32)
@@ -257,6 +290,24 @@ def convert_batch_multi(contexts, kind, argb, width, height, n_max_colors, dithe
     if rc != 0:
         raise NQuantError(rc, L.nq_last_error().decode())
     return out, pal, plen, ha
+
+
+def _palettes(palettes, n):
+    """One shared palette (a 1-D array) or one per image (a list of n of them) -> the (n_palettes, 256) uint32 array, the
+    lengths and n_palettes of the remap calls."""
+    shared = isinstance(palettes, np.ndarray) and palettes.ndim == 1
+    pals = [palettes] if shared else list(palettes)
+    if not shared and len(pals) != n:
+        raise NQuantError(_lib.NQ_ERR_ARG, "palettes: one array shared by every image, or one per image")
+    out = np.zeros((len(pals), 256), dtype=np.uint32)
+    lens = np.zeros(len(pals), dtype=np.int32)
+    for i, p in enumerate(pals):
+        p = np.asarray(p, dtype=np.uint32).reshape(-1)
+        if not 1 <= p.size <= 256:
+            raise NQuantError(_lib.NQ_ERR_ARG, f"palette {i}: length must be 1..256")
+        out[i, :p.size] = p
+        lens[i] = p.size
+    return out, lens, len(pals)
 
 
 class _Ragged:
